@@ -2,6 +2,7 @@
 """bench.py — the AV-CTC hot path on B200, next to the reference's CPU path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload train|ctc|beam|fusion|infonce]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -109,6 +110,7 @@ def build_models(device, seed=0, encoders=True):
     from multimodal_av_model_b200.encoders import unfreeze_middle_layers, xlsr_large_config
     from multimodal_av_model_b200.synthetic import CharTokenizer
     torch.manual_seed(seed)
+    np.random.seed(seed)        # wav2vec2's SpecAugment spans come from numpy's global generator: same args, same outputs
     if not encoders:
         fus = pkg.CrossAttentionFusion(512, 1024, 512)
         dec = pkg.CTCDecoder(1024, VOCAB, blank_id=BLANK)
@@ -169,6 +171,22 @@ def timed_loop(fn, steps, warmup, device, world, label=None):
     return float(ms.item())
 
 
+def dump_outputs(path, tr, loss):
+    """--dump-outputs: what the last timed train step produced, as the trainer reports it per step (train_epoch's log
+    line), so that two builds can be compared output for output: the total loss train_step returned, its four terms and
+    speaker 1's CTC log-probs [B, T, V], as <path>/{loss,ctc1,ctc2,contrastive1,contrastive2,log_probs}.npy in float32.
+    The step's gradients and updated weights are not written: the gradient reductions add float partial sums with
+    atomics, and where a gradient is only rounding noise (the attention key biases, whose exact gradient is zero) Adam
+    turns that noise into whole learning-rate steps of either sign, so they differ from run to run by more than rounding.
+    The loss terms and log-probs agree to rounding."""
+    c1, c2, k1, k2 = tr._last_parts
+    out = {"loss": loss, "ctc1": c1, "ctc2": c2, "contrastive1": k1, "contrastive2": k2,
+           "log_probs": tr._last_log_probs}
+    os.makedirs(path, exist_ok=True)
+    for k, t in out.items():
+        np.save(os.path.join(path, k + ".npy"), t.detach().float().cpu().numpy())
+
+
 def bench_train(args, rank, local, world, device, hot_only=False):
     from multimodal_av_model_b200 import _lib
     from multimodal_av_model_b200.synthetic import make_batch
@@ -178,9 +196,10 @@ def bench_train(args, rank, local, world, device, hot_only=False):
     if not hot_only:
         host = make_batch(pairs=PAIRS_PER_GPU, seconds=SECONDS, t_v=T_V, vocab=VOCAB, seed=1234 + rank, pin=True)
         dev_batch = {k: v.to(device) for k, v in host.items()}
+        last = {}
 
         def step_resident():
-            tr.train_step(dev_batch)
+            last["loss"] = tr.train_step(dev_batch)
 
         def step_e2e():
             return float(tr.train_step(host))          # H2D of the pinned batch + D2H read of the loss
@@ -189,6 +208,8 @@ def bench_train(args, rank, local, world, device, hot_only=False):
         with ClockSampler(local) as cs:
             ms = timed_loop(step_resident, args.steps, args.warmup, device, world, label="value")
         launches = (_lib.launch_count - c0) // (args.steps + args.warmup)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, tr, last["loss"])
         ms_e2e = timed_loop(step_e2e, args.steps, max(1, args.warmup // 2), device, world, label="e2e")
         # the same K steps through MultimodalTrainer.train_epoch (main.py:165): batch i+1 staged on a side stream while step i
         # runs, each step's loss sent to the pinned trainer.loss_log without blocking, one host sync at the end of the epoch
@@ -807,7 +828,13 @@ def main():
     ap.add_argument("--workload", default="train", choices=["train", "ctc", "beam", "fusion", "infonce", "lstm", "hot"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-comparators", action="store_true", help="skip the stock-torch CUDA / host CPU legs of the sub-benchmarks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss terms and log-probs of the last timed train step "
+                                                           "to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "train"):
+        ap.error("--dump-outputs needs --impl ours --workload train")
     rank = int(os.environ.get("RANK", "0"))
     if args.impl == "reference":
         run_reference(args, rank)

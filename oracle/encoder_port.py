@@ -11,8 +11,9 @@ scheduling changes: sync-free wav2vec2 forward, cast cache, channels-last), so t
   freeze policy main.py:26-31,100-106: visual encoder frozen, only wav2vec2 encoder.layers.6-9 train
 
 Sub-module names follow the reference (`frontend3D`, `trunk.layerN.i.{conv1,bn1,relu,conv2,bn2,downsample}`, `model`) so
-its state_dict loads; tests/test_oracle_golden.py::test_encoder_port_* checks both ports against the reference classes
-on CPU.  Random init only (no checkpoint is reachable offline): wav2vec2 is built from the XLSR-53-large layout.
+its state_dict loads.  Both ports were checked equal to the reference classes on CPU when written; that check needs the
+reference's source, which is not part of this repository, so the suite does not carry it.  Random init only (no
+checkpoint is reachable offline): wav2vec2 is built from the XLSR-53-large layout.
 """
 from __future__ import annotations
 

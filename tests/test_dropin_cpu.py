@@ -31,8 +31,8 @@ print("dropin ok")
 '''
 
 
-def test_dropin_shims_expose_reference_layout():
+def test_dropin_shims_expose_reference_layout(tmp_path):
     env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "dropin"), ROOT]))
-    r = subprocess.run([sys.executable, "-c", CODE], capture_output=True, text=True, env=env, cwd="/tmp")
+    r = subprocess.run([sys.executable, "-c", CODE], capture_output=True, text=True, env=env, cwd=tmp_path)
     assert r.returncode == 0, r.stderr[-2000:]
     assert "dropin ok" in r.stdout

@@ -207,61 +207,3 @@ def test_torch_port_infonce_beam_and_step_match_reference():
         if g.size:
             assert torch.allclose(prm.grad, torch.from_numpy(g), atol=2e-5), k
 
-
-# ------------------------------------------------------------------------------------------ encoder port (reference arm)
-_REF = "/root/reference"
-
-
-def _ref_encoder_module():
-    """model/encoder.py of the reference, imported in place (build container only; absent on the GPU box)."""
-    import importlib.util
-    import os
-    import sys
-    path = os.path.join(_REF, "model", "encoder.py")
-    if not os.path.exists(path):
-        pytest.skip("/root/reference is not present (GPU box)")
-    spec = importlib.util.spec_from_file_location("_ref_encoder", path)
-    mod = importlib.util.module_from_spec(spec)
-    sys.modules["_ref_encoder"] = mod
-    spec.loader.exec_module(mod)
-    return mod
-
-
-def test_encoder_port_visual_equals_reference_module():
-    import torch
-    from oracle import encoder_port as ep
-    ref_mod = _ref_encoder_module()
-    torch.manual_seed(0)
-    ref = ref_mod.VisualEncoder()
-    port = ep.VisualPort()
-    port.load_state_dict(ref.state_dict())                # same keys
-    x = torch.rand(2, 1, 7, 96, 96)
-    for mode in ("train", "eval"):
-        getattr(ref, mode)(); getattr(port, mode)()
-        assert torch.equal(ref(x), port(x))
-
-
-def test_encoder_port_audio_equals_reference_module(monkeypatch):
-    import torch
-    from transformers import Wav2Vec2Model
-    from oracle import encoder_port as ep
-    ref_mod = _ref_encoder_module()
-    cfg = ep.xlsr_large_config(num_hidden_layers=10, hidden_size=64, num_attention_heads=4, intermediate_size=128,
-                               num_conv_pos_embedding_groups=4, conv_dim=(32,) * 7)
-
-    def fake_from_pretrained(name, **kw):                 # the checkpoint needs the network: random init of the same class
-        cfg.output_hidden_states = kw.get("output_hidden_states", False)
-        return Wav2Vec2Model(cfg)
-    monkeypatch.setattr(ref_mod.Wav2Vec2Model, "from_pretrained", staticmethod(fake_from_pretrained))
-    torch.manual_seed(0)
-    ref = ref_mod.AudioEncoder(freeze=True)
-    port = ep.AudioPort(config=cfg)
-    port.load_state_dict(ref.state_dict())
-    ref.eval(); port.eval()
-    x = 0.1 * torch.randn(2, 4000)
-    m = torch.ones(2, 4000, dtype=torch.long); m[1, 3000:] = 0
-    a, mid = ref(x, attention_mask=m)
-    b, mid2 = port(x, attention_mask=m)
-    assert torch.equal(a, b) and torch.equal(mid, mid2)
-    trainable = {n for n, p in port.model.named_parameters() if p.requires_grad}
-    assert trainable and all(any(f"encoder.layers.{i}." in n for i in range(6, 10)) for n in trainable)
