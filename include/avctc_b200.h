@@ -303,6 +303,37 @@ AVCTC_API int avctc_infonce_backward(const int64_t* flat_mask, int N, int P, flo
                            const float* grad_out, void* dy, int dtype, long long ld, void* workspace,
                            size_t workspace_bytes, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Visual encoder forward (encoders.py VisualEncoder, frozen, bf16 autocast) around cuDNN's trunk convolutions.
+ * Activations are NHWC bf16 ([rows, C], C contiguous, 16-byte aligned); statistics partials are fp32 [3][C][P]
+ * (count, mean, M2 per channel and producing CTA), combined in a fixed order (bit-identical runs).
+ * avctc_visual_frontend: x [B,1,T,H,W] fp32 -> y [B*T, Ho, Wo, 64] bf16, Ho = (H-1)/2+1, Wo = (W-1)/2+1: the (5,7,7)
+ *   Conv3d, stride (1,2,2), padding (2,3,3), over the bf16-rounded clip; w_bf16 [64][256] = weight[:,0] as
+ *   [64, 5*7*7] zero-padded to 256.  partials [3][64][P], P = avctc_visual_frontend_ctas(), or NULL (no statistics).
+ * avctc_bn_stats: partials of x [M, C] (C % 8 == 0, 256 % (C/8) == 0), P = avctc_bn_stats_ctas(M, C).
+ * avctc_bn_finalize: scale_shift [2][C] = {gamma/sqrt(var+eps), beta - mean*scale}; training = 1: batch statistics
+ *   from the partials (biased variance) and running_mean/var updated in place (momentum, unbiased variance);
+ *   training = 0: from the running statistics, nothing updated.  weight / bias may be NULL (1 / 0).
+ * avctc_visual_frontend_pool: out [N, (H-1)/2+1, (W-1)/2+1, 64] = 3x3/2 max pool (padding 1) of
+ *   bf16(PReLU(bf16(y*scale+shift))), y [N, H, W, 64].
+ * avctc_bn_act: out = bf16(PReLU(z)), z = bf16(x*scale+shift) [+ residual: z = bf16(z + r), r = res or, with
+ *   res_scale_shift, bf16(res*res_scale+res_shift)]; pool_hw > 0: out [M/pool_hw, C] = bf16(mean over each
+ *   group of pool_hw rows).  slope_bf16: PReLU slope per channel.
+ * ---------------------------------------------------------------------------------------------- */
+AVCTC_API int avctc_visual_frontend_ctas(int B, int T, int H, int W);
+AVCTC_API int avctc_visual_frontend(const float* x, int B, int T, int H, int W, const void* w_bf16, void* y_bf16,
+                                    float* partials, int P, void* stream);
+AVCTC_API int avctc_bn_stats_ctas(long long M, int C);
+AVCTC_API int avctc_bn_stats(const void* x_bf16, long long M, int C, float* partials, int P, void* stream);
+AVCTC_API int avctc_bn_finalize(const float* partials, int P, int C, const float* weight, const float* bias,
+                                float* running_mean, float* running_var, float momentum, float eps, int training,
+                                float* scale_shift, void* stream);
+AVCTC_API int avctc_visual_frontend_pool(const void* y_bf16, long long N, int H, int W, const float* scale_shift,
+                                         const void* slope_bf16, void* out_bf16, void* stream);
+AVCTC_API int avctc_bn_act(const void* x_bf16, long long M, int C, const float* scale_shift, const void* slope_bf16,
+                           const void* res_bf16, const float* res_scale_shift, int pool_hw, void* out_bf16,
+                           void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -62,6 +62,13 @@ SIGNATURES = {
                                    ctypes.c_float, _vp, _vp, _sz, _vp]),
     "avctc_infonce_backward": (_i, [_vp, _i, _i, ctypes.c_float, ctypes.c_float, ctypes.c_float, _vp, _vp, _i,
                                     ctypes.c_longlong, _vp, _sz, _vp]),
+    "avctc_visual_frontend_ctas": (_i, [_i, _i, _i, _i]),
+    "avctc_visual_frontend": (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _i, _vp]),
+    "avctc_bn_stats_ctas": (_i, [ctypes.c_longlong, _i]),
+    "avctc_bn_stats": (_i, [_vp, ctypes.c_longlong, _i, _vp, _i, _vp]),
+    "avctc_bn_finalize": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, ctypes.c_float, ctypes.c_float, _i, _vp, _vp]),
+    "avctc_visual_frontend_pool": (_i, [_vp, ctypes.c_longlong, _i, _i, _vp, _vp, _vp, _vp]),
+    "avctc_bn_act": (_i, [_vp, ctypes.c_longlong, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
 }
 
 
@@ -80,7 +87,8 @@ KERNELS = {"avctc_ctc_forward": 2, "avctc_ctc_reduce": 1, "avctc_ctc_backward": 
            "avctc_softmax_backward": 1, "avctc_colsum": 1, "avctc_log_softmax_forward": 1,
            "avctc_log_softmax_backward": 1, "avctc_infonce_forward": 4, "avctc_infonce_backward": 2,
            "avctc_ctc_head_forward": 1, "avctc_ctc_head_backward": 3, "avctc_attention_forward": 1, "avctc_attention_backward": 1, "avctc_fusion_forward": 7, "avctc_fusion_backward": 8,
-           "avctc_bilstm_forward": 7, "avctc_bilstm_backward": 20}
+           "avctc_bilstm_forward": 7, "avctc_bilstm_backward": 20, "avctc_visual_frontend": 1, "avctc_bn_stats": 1,
+           "avctc_bn_finalize": 1, "avctc_visual_frontend_pool": 1, "avctc_bn_act": 1}
 launch_count = 0
 
 
