@@ -334,6 +334,53 @@ AVCTC_API int avctc_bn_act(const void* x_bf16, long long M, int C, const float* 
                            const void* res_bf16, const float* res_scale_shift, int pool_hw, void* out_bf16,
                            void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * wav2vec2 encoder layer (Wav2Vec2EncoderLayerStableLayerNorm, bf16 autocast, train or eval) around torch's attention
+ * core (csrc/wav2vec2_layer.cu).  Rows M = B*T, hidden E (multiple of 256, <= 1024), intermediate F (multiple of 8).
+ * Activations are contiguous bf16 [M, E] / [M, F], 16-byte aligned; LayerNorm weights/biases fp32; weights bf16 in
+ * nn.Linear layout; biases fp32 holding the bf16-rounded values autocast would add.  Every tensor the module path
+ * materialises in bf16 is rounded at the same point.
+ * avctc_w2v_attn_in_forward: ln1 = LayerNorm(x) (fp32 math), q/k/v = ln1 . W^T + b into three [M, E] tensors;
+ *   wqkv = [Wq; Wk; Wv] [3E, E], bqkv [3E].
+ * avctc_w2v_attn_out_ffn_forward: attn [M, E] = the attention output HF feeds out_proj; x = the layer input;
+ *   h = bf16(x + drop_h(attn . Wo^T + bo)); y = bf16(h + drop_o(drop_a(gelu(LayerNorm(h) . W1^T + b1)) . W2^T + b2)).
+ *   Dropouts (training != 0, p > 0) reproduce ATen's CUDA native_dropout for Philox (seed, offset) bit for bit; the three
+ *   take consecutive offsets from `offset` in that order, together avctc_w2v_dropout_increment(): the caller advances
+ *   its generator by that much.
+ * Backward entries take the forward's `saved` buffer unchanged plus a scratch buffer, regenerate the dropout masks from
+ *   the same (seed, offset), and write bf16 input gradients.  The fp32 parameter gradients (all NULL or all set) are
+ *   written, not accumulated; LayerNorm and bias gradients are reduced in a fixed order.
+ *   attn_in_backward: dq, dk, dv contiguous [M, E] -> dx (the LayerNorm branch's share of d x).
+ *   attn_out_ffn_backward: dy -> dattn and dx (the residual branch's share of d x).
+ * avctc_w2v_workspace_bytes: which = 0 attn_in saved, 1 attn_out_ffn saved, 2 attn_in scratch, 3 attn_out_ffn scratch.
+ * avctc_w2v_dropout: y = native_dropout(x, p) for a contiguous bf16 x of n elements (n % 8 == 0) at (seed, offset).
+ * ---------------------------------------------------------------------------------------------- */
+AVCTC_API size_t avctc_w2v_workspace_bytes(long long M, int E, int F, int which);
+AVCTC_API long long avctc_w2v_dropout_increment(long long M, int E, int F, double p_hidden, double p_act, double p_out,
+                                                int training);
+AVCTC_API int avctc_w2v_dropout(const void* x, long long n, double p, unsigned long long seed, unsigned long long offset,
+                                void* y, void* stream);
+AVCTC_API int avctc_w2v_attn_in_forward(const void* x, long long M, int E, const float* ln_w, const float* ln_b, float eps,
+                                        const void* wqkv, const float* bqkv, void* q, void* k, void* v, void* saved,
+                                        size_t saved_bytes, void* stream);
+AVCTC_API int avctc_w2v_attn_in_backward(const void* dq, const void* dk, const void* dv, const void* x, long long M, int E,
+                                         const float* ln_w, const void* wqkv, void* dx, float* g_wqkv, float* g_bqkv,
+                                         float* g_lnw, float* g_lnb, const void* saved, size_t saved_bytes, void* scratch,
+                                         size_t scratch_bytes, void* stream);
+AVCTC_API int avctc_w2v_attn_out_ffn_forward(const void* attn, const void* x, long long M, int E, int F, const void* wo,
+                                             const float* bo, const float* ln_w, const float* ln_b, float eps,
+                                             const void* w1, const float* b1, const void* w2, const float* b2,
+                                             double p_hidden, double p_act, double p_out, int training,
+                                             unsigned long long seed, unsigned long long offset, void* y, void* saved,
+                                             size_t saved_bytes, void* stream);
+AVCTC_API int avctc_w2v_attn_out_ffn_backward(const void* dy, const void* attn, long long M, int E, int F, const void* wo,
+                                              const float* ln_w, const void* w1, const void* w2, double p_hidden,
+                                              double p_act, double p_out, int training, unsigned long long seed,
+                                              unsigned long long offset, void* dattn, void* dx, float* g_wo, float* g_bo,
+                                              float* g_lnw, float* g_lnb, float* g_w1, float* g_b1, float* g_w2,
+                                              float* g_b2, const void* saved, size_t saved_bytes, void* scratch,
+                                              size_t scratch_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

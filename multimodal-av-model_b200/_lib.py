@@ -17,6 +17,7 @@ F32, BF16 = 0, 1
 REDUCTION = {"none": 0, "mean": 1, "sum": 2}
 
 _vp, _i, _i64, _sz = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_size_t
+_d, _u64 = ctypes.c_double, ctypes.c_uint64
 
 # name -> (restype, argtypes); must list every symbol include/avctc_b200.h declares
 SIGNATURES = {
@@ -69,6 +70,17 @@ SIGNATURES = {
     "avctc_bn_finalize": (_i, [_vp, _i, _i, _vp, _vp, _vp, _vp, ctypes.c_float, ctypes.c_float, _i, _vp, _vp]),
     "avctc_visual_frontend_pool": (_i, [_vp, ctypes.c_longlong, _i, _i, _vp, _vp, _vp, _vp]),
     "avctc_bn_act": (_i, [_vp, ctypes.c_longlong, _i, _vp, _vp, _vp, _vp, _i, _vp, _vp]),
+    "avctc_w2v_workspace_bytes": (_sz, [ctypes.c_longlong, _i, _i, _i]),
+    "avctc_w2v_dropout_increment": (ctypes.c_longlong, [ctypes.c_longlong, _i, _i, _d, _d, _d, _i]),
+    "avctc_w2v_dropout": (_i, [_vp, ctypes.c_longlong, _d, _u64, _u64, _vp, _vp]),
+    "avctc_w2v_attn_in_forward": (_i, [_vp, ctypes.c_longlong, _i, _vp, _vp, ctypes.c_float, _vp, _vp, _vp, _vp, _vp,
+                                       _vp, _sz, _vp]),
+    "avctc_w2v_attn_in_backward": (_i, [_vp, _vp, _vp, _vp, ctypes.c_longlong, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                        _vp, _sz, _vp, _sz, _vp]),
+    "avctc_w2v_attn_out_ffn_forward": (_i, [_vp, _vp, ctypes.c_longlong, _i, _i, _vp, _vp, _vp, _vp, ctypes.c_float,
+                                            _vp, _vp, _vp, _vp, _d, _d, _d, _i, _u64, _u64, _vp, _vp, _sz, _vp]),
+    "avctc_w2v_attn_out_ffn_backward": (_i, [_vp, _vp, ctypes.c_longlong, _i, _i, _vp, _vp, _vp, _vp, _d, _d, _d, _i,
+                                             _u64, _u64, _vp, _vp] + [_vp] * 8 + [_vp, _sz, _vp, _sz, _vp]),
 }
 
 
@@ -88,7 +100,12 @@ KERNELS = {"avctc_ctc_forward": 2, "avctc_ctc_reduce": 1, "avctc_ctc_backward": 
            "avctc_log_softmax_backward": 1, "avctc_infonce_forward": 4, "avctc_infonce_backward": 2,
            "avctc_ctc_head_forward": 1, "avctc_ctc_head_backward": 3, "avctc_attention_forward": 1, "avctc_attention_backward": 1, "avctc_fusion_forward": 7, "avctc_fusion_backward": 8,
            "avctc_bilstm_forward": 7, "avctc_bilstm_backward": 20, "avctc_visual_frontend": 1, "avctc_bn_stats": 1,
-           "avctc_bn_finalize": 1, "avctc_visual_frontend_pool": 1, "avctc_bn_act": 1}
+           "avctc_bn_finalize": 1, "avctc_visual_frontend_pool": 1, "avctc_bn_act": 1, "avctc_w2v_dropout": 1,
+           "avctc_w2v_attn_in_forward": 2, "avctc_w2v_attn_out_ffn_forward": 6, "avctc_w2v_attn_in_backward": 3,
+           "avctc_w2v_attn_out_ffn_backward": 6}
+# wav2vec2 layer backward: 2 more kernels (bias / LayerNorm gradient reductions) when the weight-gradient pointer at this
+# argument index is set
+_WGRAD_ARG = {"avctc_w2v_attn_in_backward": 9, "avctc_w2v_attn_out_ffn_backward": 17}
 launch_count = 0
 
 
@@ -110,6 +127,13 @@ class _Counted:
             def call(*a):
                 global launch_count
                 launch_count += 2 if route(a[3], a[4], a[5], a[7]) == 2 else 1
+                return fn(*a)
+        elif name in _WGRAD_ARG:
+            arg = _WGRAD_ARG[name]
+
+            def call(*a):
+                global launch_count
+                launch_count += n + (2 if a[arg] else 0)
                 return fn(*a)
         else:
             def call(*a):

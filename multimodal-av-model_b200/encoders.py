@@ -1,6 +1,8 @@
 """Producers that feed the hot path: VisualEncoder and AudioEncoder (SURVEY.md §8 row a15).
 
-The third-party wav2vec2 stays HF/PyTorch.  The frozen visual encoder's bf16-autocast forward on CUDA runs on this
+The third-party wav2vec2 stays HF/PyTorch except for its encoder layers that a gradient flows through: on CUDA under bf16
+autocast those run on this library's kernels (csrc/wav2vec2_layer.cu) around torch's attention core, with dropout
+identical to ATen's; the module path is the CPU path and the reference.  The frozen visual encoder's bf16-autocast forward on CUDA runs on this
 library's kernels (csrc/visual_encoder.cu: front end, BatchNorm, PReLU, residual and pooling passes) around cuDNN's trunk
 convolutions; its module path is the CPU path and the reference the tests compare against.  Module and
 parameter names follow /root/reference/model/encoder.py:6-100 so reference checkpoints load unchanged
@@ -397,12 +399,211 @@ class AudioEncoder(nn.Module):
                 seg = self._layer_segment(layer)
                 if seg.usable(hidden, mask4d):      # frozen layer, no gradient flows through it yet (layers 0-5 in
                     hidden = seg(hidden, mask4d)    # training, every frozen layer under no_grad): one graph launch
+                elif _w2v_native_applies(layer, hidden):
+                    hidden = _w2v_native_layer(layer, hidden, mask4d)
                 else:
                     hidden = layer(hidden, attention_mask=mask4d, output_attentions=False)[0]
         if stable:
             hidden = enc.layer_norm(hidden)
         all_hidden = all_hidden + (hidden,)
         return hidden, all_hidden
+
+
+# ------------------------------------------------------------------------------------ native wav2vec2 layers
+# The layers a gradient flows through (6-9 train, 10-23 carry the input gradient back to them) cannot be graphed; through
+# HF's module code each layer-call costs ~100 dispatcher ops forward and 80-144 backward, and the host's enqueue of them
+# bounded the train step.  On the native path a layer is two library calls per direction (csrc/wav2vec2_layer.cu) with
+# torch's attention interface between them, called exactly as Wav2Vec2Attention.forward calls it (its dropout stream
+# cannot be reproduced by our own kernel).  The module path stays the reference and the path for everything else.
+
+def _w2v_native_applies(layer, hidden):
+    """bf16-autocast CUDA forward of a Wav2Vec2EncoderLayerStableLayerNorm with sdpa attention, exact GELU, no adapter,
+    fp32 parameters and dropout probabilities below 1, outside stream capture."""
+    from transformers.models.wav2vec2.modeling_wav2vec2 import Wav2Vec2EncoderLayerStableLayerNorm
+    if not (hidden.is_cuda and hidden.dtype == torch.bfloat16 and hidden.dim() == 3 and hidden.is_contiguous()
+            and torch.is_autocast_enabled("cuda") and torch.get_autocast_dtype("cuda") == torch.bfloat16
+            and not torch.cuda.is_current_stream_capturing()):
+        return False
+    if type(layer) is not Wav2Vec2EncoderLayerStableLayerNorm or layer.adapter_layer is not None:
+        return False
+    cfg = layer.attention.config
+    if getattr(cfg, "_attn_implementation", None) != "sdpa" or cfg.hidden_act != "gelu":
+        return False
+    e, f = hidden.shape[-1], layer.feed_forward.intermediate_dense.out_features
+    if e % 256 or e > 1024 or f % 8 or hidden.shape[0] * hidden.shape[1] == 0:
+        return False
+    ff = layer.feed_forward
+    if any(not 0.0 <= d.p < 1.0 for d in (layer.dropout, ff.intermediate_dropout, ff.output_dropout)):
+        return False
+    return all(p.dtype == torch.float32 and p.is_cuda for p in layer.parameters())
+
+
+_optimizer_steps = [0]
+_optimizer_hook = []
+
+
+def _optimizer_step_count():
+    """torch.optim steps taken in this process since the first call.  Adam(fused=True) updates parameters in place without
+    advancing their version counters, so a version key alone would keep serving the weights of before the step."""
+    if not _optimizer_hook:
+        from torch.optim.optimizer import register_optimizer_step_post_hook
+
+        def bump(opt, args, kwargs):
+            _optimizer_steps[0] += 1
+        _optimizer_hook.append(register_optimizer_step_post_hook(bump))
+    return _optimizer_steps[0]
+
+
+def _w2v_params(layer):
+    """bf16 weight copies the kernels read and the bf16-rounded biases autocast would add, made once per parameter
+    version: frozen layers cast once, trainable ones once per optimizer step (shared by both calls of the step)."""
+    a, ff = layer.attention, layer.feed_forward
+    lins = (a.q_proj, a.k_proj, a.v_proj, a.out_proj, ff.intermediate_dense, ff.output_dense)
+    params = [p for m in lins for p in (m.weight, m.bias)]
+    steps = _optimizer_step_count() if any(p.requires_grad for p in params) else None
+    key = (steps, tuple((p._version, p.data_ptr()) for p in params))
+    hit = getattr(layer, "_avctc_w2v_cache", None)
+    if hit is None or hit[0] != key:
+        bf = torch.bfloat16
+        with torch.no_grad():
+            prm = {"wqkv": torch.cat([a.q_proj.weight, a.k_proj.weight, a.v_proj.weight]).to(bf),
+                   "bqkv": torch.cat([a.q_proj.bias, a.k_proj.bias, a.v_proj.bias]).to(bf).float(),
+                   "wo": a.out_proj.weight.to(bf), "bo": a.out_proj.bias.to(bf).float(),
+                   "w1": ff.intermediate_dense.weight.to(bf), "b1": ff.intermediate_dense.bias.to(bf).float(),
+                   "w2": ff.output_dense.weight.to(bf), "b2": ff.output_dense.bias.to(bf).float()}
+        hit = (key, prm)
+        object.__setattr__(layer, "_avctc_w2v_cache", hit)
+    return hit[1]
+
+
+class _W2VAttnIn(torch.autograd.Function):
+    """q, k, v = projections of LayerNorm(x): avctc_w2v_attn_in_forward / _backward."""
+
+    @staticmethod
+    def forward(ctx, x, ln_w, ln_b, wq, bq, wk, bk, wv, bv, prm, eps):
+        from . import _lib
+        L = _lib.lib()
+        b, t, e = x.shape
+        m = b * t
+        with _lib.device_guard(x.device):
+            saved = torch.empty(L.avctc_w2v_workspace_bytes(m, e, 8, 0), dtype=torch.uint8, device=x.device)
+            q, k, v = torch.empty_like(x), torch.empty_like(x), torch.empty_like(x)
+            _lib.check(L.avctc_w2v_attn_in_forward(x.data_ptr(), m, e, ln_w.data_ptr(), ln_b.data_ptr(), eps,
+                                                   prm["wqkv"].data_ptr(), prm["bqkv"].data_ptr(), q.data_ptr(),
+                                                   k.data_ptr(), v.data_ptr(), saved.data_ptr(), saved.numel(),
+                                                   _lib.stream_ptr(x.device)), "avctc_w2v_attn_in_forward")
+        ctx.save_for_backward(x, ln_w, saved)
+        ctx.prm = prm
+        return q, k, v
+
+    @staticmethod
+    def backward(ctx, dq, dk, dv):
+        from . import _lib
+        L = _lib.lib()
+        x, ln_w, saved = ctx.saved_tensors
+        b, t, e = x.shape
+        m, dev = b * t, x.device
+        need = ctx.needs_input_grad
+        wg = any(need[1:9])
+        dq, dk, dv = (g.to(torch.bfloat16).contiguous() for g in (dq, dk, dv))
+        with _lib.device_guard(dev):
+            scratch = torch.empty(L.avctc_w2v_workspace_bytes(m, e, 8, 2), dtype=torch.uint8, device=dev)
+            dx = torch.empty_like(x)
+            g = [None] * 4
+            if wg:
+                g = [torch.empty((3 * e, e), device=dev), torch.empty(3 * e, device=dev), torch.empty(e, device=dev),
+                     torch.empty(e, device=dev)]
+            _lib.check(L.avctc_w2v_attn_in_backward(dq.data_ptr(), dk.data_ptr(), dv.data_ptr(), x.data_ptr(), m, e,
+                                                    ln_w.data_ptr(), ctx.prm["wqkv"].data_ptr(), dx.data_ptr(),
+                                                    *[a.data_ptr() if a is not None else None for a in g],
+                                                    saved.data_ptr(), saved.numel(), scratch.data_ptr(), scratch.numel(),
+                                                    _lib.stream_ptr(dev)), "avctc_w2v_attn_in_backward")
+        if not wg:
+            return dx, None, None, None, None, None, None, None, None, None, None
+        gw, gb, glw, glb = g
+        out = [glw, glb, gw[:e], gb[:e], gw[e:2 * e], gb[e:2 * e], gw[2 * e:], gb[2 * e:]]
+        return (dx, *[o if n else None for o, n in zip(out, need[1:9])], None, None)
+
+
+class _W2VAttnOutFFN(torch.autograd.Function):
+    """out_proj, hidden dropout, residual, final LayerNorm, feed-forward with its two dropouts, residual:
+    avctc_w2v_attn_out_ffn_forward / _backward.  The three dropouts take their generator offsets here, after the
+    attention core took its own, in module order."""
+
+    @staticmethod
+    def forward(ctx, attn, x, wo, bo, ln_w, ln_b, w1, b1, w2, b2, prm, eps, probs):
+        from . import _lib
+        L = _lib.lib()
+        b, t, e = x.shape
+        m, f, dev = b * t, w1.shape[0], x.device
+        with _lib.device_guard(dev):
+            incr = L.avctc_w2v_dropout_increment(m, e, f, *probs, 1)
+            _lib.check(0 if incr >= 0 else incr, "avctc_w2v_dropout_increment")
+            seed = offset = 0
+            if incr:
+                gen = torch.cuda.default_generators[dev.index]
+                seed, offset = gen.initial_seed(), gen.get_offset()
+                gen.set_offset(offset + incr)
+            saved = torch.empty(L.avctc_w2v_workspace_bytes(m, e, f, 1), dtype=torch.uint8, device=dev)
+            y = torch.empty_like(x)
+            _lib.check(L.avctc_w2v_attn_out_ffn_forward(attn.data_ptr(), x.data_ptr(), m, e, f, prm["wo"].data_ptr(),
+                                                        prm["bo"].data_ptr(), ln_w.data_ptr(), ln_b.data_ptr(), eps,
+                                                        prm["w1"].data_ptr(), prm["b1"].data_ptr(), prm["w2"].data_ptr(),
+                                                        prm["b2"].data_ptr(), *probs, 1, seed, offset, y.data_ptr(),
+                                                        saved.data_ptr(), saved.numel(), _lib.stream_ptr(dev)),
+                       "avctc_w2v_attn_out_ffn_forward")
+        wg = any(ctx.needs_input_grad[2:10])
+        ctx.save_for_backward(attn if wg else None, ln_w, saved)
+        ctx.prm, ctx.probs, ctx.seed, ctx.offset, ctx.dims = prm, probs, seed, offset, (b, t, e, f)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        from . import _lib
+        L = _lib.lib()
+        attn, ln_w, saved = ctx.saved_tensors
+        b, t, e, f = ctx.dims
+        m, dev = b * t, ln_w.device
+        need = ctx.needs_input_grad
+        wg = any(need[2:10])
+        dy = dy.to(torch.bfloat16).contiguous()
+        prm = ctx.prm
+        with _lib.device_guard(dev):
+            scratch = torch.empty(L.avctc_w2v_workspace_bytes(m, e, f, 3), dtype=torch.uint8, device=dev)
+            dattn, dx = torch.empty_like(dy), torch.empty_like(dy)
+            g = [None] * 8
+            if wg:
+                g = [torch.empty((e, e), device=dev), torch.empty(e, device=dev), torch.empty(e, device=dev),
+                     torch.empty(e, device=dev), torch.empty((f, e), device=dev), torch.empty(f, device=dev),
+                     torch.empty((e, f), device=dev), torch.empty(e, device=dev)]
+            _lib.check(L.avctc_w2v_attn_out_ffn_backward(
+                dy.data_ptr(), attn.data_ptr() if attn is not None else dy.data_ptr(), m, e, f, prm["wo"].data_ptr(),
+                ln_w.data_ptr(), prm["w1"].data_ptr(), prm["w2"].data_ptr(), *ctx.probs, 1, ctx.seed, ctx.offset,
+                dattn.data_ptr(), dx.data_ptr(), *[a.data_ptr() if a is not None else None for a in g],
+                saved.data_ptr(), saved.numel(), scratch.data_ptr(), scratch.numel(), _lib.stream_ptr(dev)),
+                "avctc_w2v_attn_out_ffn_backward")
+        return (dattn, dx, *[o if n else None for o, n in zip(g, need[2:10])], None, None, None)
+
+
+def _w2v_native_layer(layer, hidden, mask4d):
+    """Wav2Vec2EncoderLayerStableLayerNorm.forward(hidden, attention_mask=mask4d)[0] on the native path."""
+    from transformers.modeling_utils import ALL_ATTENTION_FUNCTIONS
+    from transformers.models.wav2vec2.modeling_wav2vec2 import eager_attention_forward
+    a, ff = layer.attention, layer.feed_forward
+    ln1, ln2 = layer.layer_norm, layer.final_layer_norm
+    prm = _w2v_params(layer)
+    b, t, _ = hidden.shape
+    q, k, v = _W2VAttnIn.apply(hidden, ln1.weight, ln1.bias, a.q_proj.weight, a.q_proj.bias, a.k_proj.weight,
+                               a.k_proj.bias, a.v_proj.weight, a.v_proj.bias, prm, ln1.eps)
+    shape = (b, t, -1, a.head_dim)
+    interface = ALL_ATTENTION_FUNCTIONS.get_interface(a.config._attn_implementation, eager_attention_forward)
+    o, _ = interface(a, q.view(shape).transpose(1, 2), k.view(shape).transpose(1, 2), v.view(shape).transpose(1, 2),
+                     mask4d, dropout=0.0 if not a.training else a.dropout, scaling=a.scaling, output_attentions=False)
+    o = o.reshape(b, t, -1).contiguous()
+    probs = tuple(float(d.p) if d.training else 0.0 for d in (layer.dropout, ff.intermediate_dropout, ff.output_dropout))
+    return _W2VAttnOutFFN.apply(o, hidden, a.out_proj.weight, a.out_proj.bias, ln2.weight, ln2.bias,
+                                ff.intermediate_dense.weight, ff.intermediate_dense.bias, ff.output_dense.weight,
+                                ff.output_dense.bias, prm, ln2.eps, probs)
 
 
 def _to_device_async(t, device):
