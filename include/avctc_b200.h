@@ -122,6 +122,28 @@ AVCTC_API int avctc_ctc_scale_grad(void* grad, int dtype, int T, int B, int V, c
                          int64_t grad_out_stride, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * CTC forced alignment — torchaudio.functional.forced_align (Viterbi over the CTC lattice) for a padded batch
+ * log_probs: utterance n, frame t, class c at log_probs[n*stride_n + t*stride_t + c] (fp32 or bf16 per dtype,
+ * class stride 1; the [T,N,V] view the CTC loss takes is stride_n = V, stride_t = N*V).  targets int64, utterance
+ * n's labels at targets[n*target_stride ..]; input_lengths / target_lengths are int64 DEVICE tensors read on the
+ * device (no host sync).
+ * Outputs (caller-owned, written for every utterance): paths[n*T + t] (int32) = the label aligned to frame t,
+ * scores[n*T + t] (log_probs dtype) = log_probs of that label at frame t, an exact copy; frames t >= input_lengths[n]
+ * get blank and 0.  status[n] (int32): 0 aligned; 1 a label among the first target_lengths[n] is blank or outside
+ * [0,V); 2 infeasible: input_lengths[n] < L + R (R = adjacent repeats); 3 a length outside [0,T] / [0,max_target_len].
+ * A non-zero status leaves the row blank / 0.  Results are bit-identical to torchaudio's CPU forced_align run on the
+ * utterance alone (same float32 sums, same comparison order on ties).  target_lengths[n] = 0 aligns every frame to
+ * blank (torchaudio cannot express it).
+ * Supported: 2*max_target_len+1 <= 511 and T x 128 bytes of back-pointers in shared memory (T up to ~1700);
+ * AVCTC_ERR_UNSUPPORTED otherwise.  avctc_ctc_align_supported is the host-side query (1 = supported, 0 = not).
+ * ---------------------------------------------------------------------------------------------- */
+AVCTC_API int avctc_ctc_align_supported(int T, int max_target_len);
+AVCTC_API int avctc_ctc_align(const void* log_probs, int dtype, int64_t stride_n, int64_t stride_t, int N, int T, int V,
+                    const int64_t* targets, int64_t target_stride, const int64_t* input_lengths,
+                    const int64_t* target_lengths, int max_target_len, int blank, int32_t* paths, void* scores,
+                    int32_t* status, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Beam-search decode — replaces simple_beam_search(log_probs[T,V], beam_width, blank)
  *   /root/reference/beam_search.py:2-42, called per utterance at model/trainer.py:230,237
  * Batched: one CTA per utterance.  log_probs fp32, utterance n frame t class c at

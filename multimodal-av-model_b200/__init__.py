@@ -9,6 +9,7 @@ hyphen).  Public names mirror the reference modules (SURVEY.md §8b):
     contrastive_loss_with_mask                contrastive.py
     simple_beam_search, fast_decode           beam_search.py  (+ beam_search_batch)
     MultimodalTrainer                         model/trainer.py
+    forced_align, merge_tokens, TokenSpan     torchaudio.functional's CTC forced alignment, batched (align.py)
 """
 from . import _lib
 from .ctc import CTCLoss, ctc_loss
@@ -28,5 +29,6 @@ _optional("beam_search", ["simple_beam_search", "fast_decode", "beam_search_batc
 _optional("fusion_module", ["CrossAttentionFusion"])
 _optional("decoder", ["CTCDecoder"])
 _optional("contrastive", ["contrastive_loss_with_mask"])
+_optional("align", ["forced_align", "merge_tokens", "merge_tokens_batch", "TokenSpan"])
 _optional("trainer", ["MultimodalTrainer"])
 _optional("encoders", ["VisualEncoder", "AudioEncoder"])

@@ -33,6 +33,8 @@ SIGNATURES = {
     "avctc_ctc_forward_backward": (_i, [_vp, _i, _i64, _i64, _i, _i, _i, _vp, _i64, _vp, _vp, _vp, _i, _i, _i, _i,
                                         _vp, _vp, _vp, _i64, _vp, _vp, _sz, _vp]),
     "avctc_ctc_scale_grad": (_i, [_vp, _i, _i, _i, _i, _vp, _i64, _vp]),
+    "avctc_ctc_align_supported": (_i, [_i, _i]),
+    "avctc_ctc_align": (_i, [_vp, _i, _i64, _i64, _i, _i, _i, _vp, _i64, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     "avctc_beam_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "avctc_beam_route": (_i, [_i, _i, _i, _i]),
     "avctc_beam_search": (_i, [_vp, _i64, _i64, _i, _i, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
@@ -94,7 +96,7 @@ class GemmOperand(ctypes.Structure):
 
 # kernels launched by each entry point (bench.py reports "gpu_launches" from this table); CTC forward / backward with a
 # workspace = the probability-domain kernel + its guarded log-domain twin (which exits at once unless the range guard tripped)
-KERNELS = {"avctc_ctc_forward": 2, "avctc_ctc_reduce": 1, "avctc_ctc_backward": 2, "avctc_ctc_forward_backward": 5, "avctc_ctc_scale_grad": 1, "avctc_beam_search": 2,
+KERNELS = {"avctc_ctc_forward": 2, "avctc_ctc_reduce": 1, "avctc_ctc_backward": 2, "avctc_ctc_forward_backward": 5, "avctc_ctc_scale_grad": 1, "avctc_ctc_align": 1, "avctc_beam_search": 2,
            "avctc_gemm_bf16": 1, "avctc_resample_forward": 2, "avctc_resample_backward": 1, "avctc_softmax_forward": 1,
            "avctc_softmax_backward": 1, "avctc_colsum": 1, "avctc_log_softmax_forward": 1,
            "avctc_log_softmax_backward": 1, "avctc_infonce_forward": 4, "avctc_infonce_backward": 2,

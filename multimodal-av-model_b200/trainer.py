@@ -6,6 +6,7 @@ Same constructor, attributes and methods (SURVEY.md §8b):
                       learning_rate=1e-4, device="cuda", lambda_=0.1)
     .train_epoch(dataloader) -> float          .evaluate(dataloader) -> (avg_loss, avg_wer)
     .ctc_decode(pred_ids)                      .crop_or_pad_feat(feat, target_len)
+    .align(batch) -> token time spans of both speakers' reference transcripts (not in the reference; CTC forced alignment)
     attributes: visual_encoder audio_encoder fusion_module decoder1 tokenizer optimizer device lambda_ ctc_loss
 
 Differences that matter (all deliberate, none changes a result):
@@ -27,6 +28,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import _lib
+from .align import TimedTokenSpan, forced_align, fused_frame_encoder_index, merge_tokens_batch
 from .beam_search import beam_search_batch, fast_decode
 from .contrastive import contrastive_loss_with_mask
 from .ctc import CTCLoss
@@ -439,3 +441,55 @@ class MultimodalTrainer:
         if self.verbose:
             print(f"[Eval] WER1: {wer1:.3f}, WER2: {wer2:.3f}, Avg: {avg_wer:.3f}, Loss: {avg_loss:.4f}")
         return avg_loss, avg_wer
+
+    # ------------------------------------------------------------------------------------------ alignment
+    hop_seconds = 320 / 16000                 # wav2vec2 encoder frame hop at 16 kHz
+
+    def align(self, batch):
+        """Who said what, when: force-aligns each speaker's reference transcript (text{s}, text{s}_lengths) to the CTC
+        head's log-probs, computed in eval mode with the encoder -> fusion -> decoder1 path the training loss sees, one
+        forced_align call per speaker.  Returns spans[s][b] = list of TimedTokenSpan, one per target token: frames of
+        the fused sequence [start, end), the piece text, and [start_sec, end_sec] in the mixed recording.
+
+        The fused sequence is not wall-clock: the fusion compacts the speaker's speech frames and resamples them to T_v.
+        Fused frame f maps to speech-frame rank nearest_src_index(T_v, Tp)[f] (Tp = the batch's largest speech-frame
+        count), that rank to its encoder frame k, and k to k * hop_seconds; a span covers [sec(k_start),
+        sec(k_{end-1}) + hop_seconds].  Raises (forced_align) if a transcript is too long for its input length."""
+        for m in (self.visual_encoder, self.audio_encoder, self.fusion_module, self.decoder1):
+            m.eval()
+        blank = self.tokenizer.blank_id
+        res = []
+        with torch.no_grad():
+            if hasattr(self.audio_encoder, "begin_step"):
+                self.audio_encoder.begin_step()
+            d = self._to_dev(batch)
+            with torch.autocast("cuda", dtype=self.autocast_dtype, enabled=str(self.device).startswith("cuda")):
+                for s in range(2):
+                    vis = self.visual_encoder(d["lips"][s]())
+                    aud, _ = self.audio_encoder(d["audio"], attention_mask=(d["masks"][s] != 3))
+                    t_enc = aud.shape[1]
+                    mask_ds = F.interpolate(d["masks"][s].unsqueeze(1).float(), size=t_enc, mode="nearest").squeeze(1).long()
+                    fused, il = self.fusion_module(vis, aud, mask_ds)
+                    lp = self.decoder1(fused)
+                    paths, scores = forced_align(lp, d["texts"][s], il, d["lens"][s], blank=blank)
+                    res.append((merge_tokens_batch(paths, scores, il, blank=blank),
+                                fused_frame_encoder_index(mask_ds.cpu(), lp.shape[1])))
+        out = []
+        for spans, enc in res:
+            spk = []
+            for b, row in enumerate(spans):
+                k = enc[b].tolist()
+                spk.append([TimedTokenSpan(token=sp.token, start=sp.start, end=sp.end, score=sp.score,
+                                           piece=self._piece(sp.token), start_sec=k[sp.start] * self.hop_seconds,
+                                           end_sec=k[sp.end - 1] * self.hop_seconds + self.hop_seconds)
+                            for sp in row])
+            out.append(spk)
+        return out
+
+    def _piece(self, token):
+        tok = self.tokenizer
+        if hasattr(tok, "id_to_piece"):
+            return tok.id_to_piece(token)
+        if hasattr(tok, "id_to_token"):
+            return tok.id_to_token[token]
+        return tok.decode([token])
