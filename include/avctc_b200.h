@@ -168,6 +168,24 @@ AVCTC_API int avctc_beam_search(const float* log_probs, int64_t stride_n, int64_
                       void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * CTC prefix beam search with N-best hypotheses (csrc/ctc_prefix_beam.cu; the search is defined in DESIGN.md §4.13 and
+ * restated in oracle/prefix_beam_oracle.py, whose results it reproduces bit for bit).  Prefixes are scored by the
+ * probability of all their alignments (fp64 natural logs).  log_probs fp32, utterance n frame t class c at
+ * log_probs[n*stride_n + t*stride_t + c]; lengths int64 device (NULL = all T frames), read on the device.
+ * beam in 1..15, nbest in 1..beam, blank in [0,V); V <= 1024 (AVCTC_ERR_UNSUPPORTED otherwise).
+ * Outputs: hypothesis i of utterance n (best first) has out_len[n*nbest + i] tokens at out_tokens[(n*nbest + i)*T ..]
+ * (entries past out_len are left untouched) and log-probability out_scores[n*nbest + i] (double).  Unused slots get
+ * length 0 and score -inf.  status[n] (int32): 0 decoded; 1 a frame's log-probs contain NaN; 2 lengths[n] outside [0,T].
+ * A failed utterance has no hypotheses.  lengths[n] = 0 gives one empty hypothesis of score 0.
+ * Two kernel launches, no host sync.  The workspace query returns 0 for an unsupported shape.
+ * ---------------------------------------------------------------------------------------------- */
+AVCTC_API size_t avctc_ctc_prefix_beam_workspace_bytes(int N, int T, int V, int beam);
+AVCTC_API int avctc_ctc_prefix_beam(const float* log_probs, int64_t stride_n, int64_t stride_t, int N, int T, int V,
+                                    const int64_t* lengths, int beam, int nbest, int blank, int32_t* out_tokens,
+                                    int32_t* out_len, double* out_scores, int32_t* status, void* workspace,
+                                    size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Fusion path dense contraction (tcgen05 + TMEM + TMA) — replaces the cuBLAS GEMMs under
  *   nn.Linear x4            /root/reference/model/fusion_module.py:57,58,63; model/decoder.py:24
  *   nn.MultiheadAttention   /root/reference/model/fusion_module.py:61 (in/out projections, Q.K^T, P.V)

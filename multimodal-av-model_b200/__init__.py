@@ -10,6 +10,7 @@ hyphen).  Public names mirror the reference modules (SURVEY.md §8b):
     simple_beam_search, fast_decode           beam_search.py  (+ beam_search_batch)
     MultimodalTrainer                         model/trainer.py
     forced_align, merge_tokens, TokenSpan     torchaudio.functional's CTC forced alignment, batched (align.py)
+    ctc_prefix_beam_search, Hypothesis        CTC prefix beam search with N-best hypotheses and scores (prefix_beam.py)
 """
 from . import _lib
 from .ctc import CTCLoss, ctc_loss
@@ -30,5 +31,6 @@ _optional("fusion_module", ["CrossAttentionFusion"])
 _optional("decoder", ["CTCDecoder"])
 _optional("contrastive", ["contrastive_loss_with_mask"])
 _optional("align", ["forced_align", "merge_tokens", "merge_tokens_batch", "TokenSpan"])
+_optional("prefix_beam", ["ctc_prefix_beam_search", "Hypothesis"])
 _optional("trainer", ["MultimodalTrainer"])
 _optional("encoders", ["VisualEncoder", "AudioEncoder"])

@@ -24,6 +24,7 @@
 // candidates can survive the prune (every (b',j') <= (b,j) sorts first), so <= ~beam*ln(beam) candidates are ranked by
 // counting, scores in fp64, back-pointers kept per frame.
 #include "common.cuh"
+#include "beam_internal.h"
 
 namespace avctc {
 
@@ -1075,9 +1076,59 @@ static int beam_sm_count() {
     return sms;
 }
 
+// beam_topk_kernel over all N*T rows (V <= 1024, N*T < 2^31): bp.beam entries per row into bp.tk_val / bp.tk_idx
+static int topk_launch(const BeamParams& bp, size_t smem_topk, int sms, cudaStream_t st) {
+    const int V = bp.V;
+    const int need = (V + 31) / 32;
+    long long blocks = ((long long)bp.N * bp.T + kTopkWarps - 1) / kTopkWarps;
+    if (blocks > (long long)sms * 8) blocks = (long long)sms * 8;
+    if (blocks < 1) blocks = 1;
+#define AVCTC_TOPK(NV, MODE)                                                                                        \
+    do {                                                                                                            \
+        static bool cfg = false;                                                                                    \
+        if (!cfg && smem_topk > 48 * 1024) {                                                                        \
+            AVCTC_CUDA_RETURN(cudaFuncSetAttribute(beam_topk_kernel<NV, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                                   200 * 1024));                                                    \
+            cfg = true;                                                                                             \
+        }                                                                                                           \
+        beam_topk_kernel<NV, MODE><<<(unsigned)blocks, kTopkWarps * 32, smem_topk, st>>>(bp);                       \
+    } while (0)
+#define AVCTC_TOPK_M(NV)                                                                                            \
+    do {                                                                                                            \
+        if (V == 32 * NV) AVCTC_TOPK(NV, 0);                                                                        \
+        else if (V > 32 * (NV - 1)) AVCTC_TOPK(NV, 1);                                                              \
+        else AVCTC_TOPK(NV, 2);                                                                                     \
+    } while (0)
+    if (need <= 4) AVCTC_TOPK(4, 2);
+    else if (need <= 8) AVCTC_TOPK(8, 2);
+    else if (need <= 16) AVCTC_TOPK(16, 2);
+    else if (need <= 25) AVCTC_TOPK_M(25);
+    else if (need <= 26) AVCTC_TOPK_M(26);
+    else AVCTC_TOPK_M(32);
+#undef AVCTC_TOPK_M
+#undef AVCTC_TOPK
+    return (int)cudaGetLastError();
+}
+
 }  // namespace avctc
 
 using namespace avctc;
+
+int avctc_beam_topk_lists(const float* log_probs, int64_t stride_n, int64_t stride_t, int N, int T, int V,
+                          const int64_t* lengths, int k, float* tk_val, int32_t* tk_idx, void* stream) {
+    if (N < 0 || T < 0 || V < 1 || V > 1024 || k < 1 || k + 1 > 32 || k > V) return AVCTC_ERR_UNSUPPORTED;
+    if ((long long)N * T >= (1ll << 31)) return AVCTC_ERR_UNSUPPORTED;
+    BeamParams bp = {};
+    bp.lp = log_probs; bp.stride_n = stride_n; bp.stride_t = stride_t;
+    bp.N = N; bp.T = T; bp.V = V; bp.lengths = lengths; bp.beam = k;
+    bp.fast = avctc_tuning_get("beam_fast", 1);
+    bp.prefetch = avctc_tuning_get("beam_pf", 1);
+    bp.row_floats = (V + 8 + 3) & ~3;
+    bp.use_nth = ((long long)k * 64 > V) ? 1 : 0;
+    bp.tk_val = tk_val; bp.tk_idx = tk_idx;
+    return topk_launch(bp, (size_t)kTopkWarps * topk_smem_per_warp(bp.row_floats, bp.use_nth), beam_sm_count(),
+                       reinterpret_cast<cudaStream_t>(stream));
+}
 
 extern "C" int avctc_beam_route(int N, int T, int V, int beam) {
     BeamPlan pl;
@@ -1127,8 +1178,6 @@ extern "C" int avctc_beam_search(const float* log_probs, int64_t stride_n, int64
         bp.tk_idx = reinterpret_cast<int32_t*>(w + pl.off_ti);
         bp.bp_global = pl.bp_in_smem2 ? nullptr : reinterpret_cast<uint32_t*>(w + pl.off_bp);
         const int need = (V + 31) / 32;
-        const long long rows = (long long)N * T;
-        long long blocks = (rows + kTopkWarps - 1) / kTopkWarps;
         int dev = 0, sms = 148;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -1144,32 +1193,8 @@ extern "C" int avctc_beam_search(const float* log_probs, int64_t stride_n, int64
             }
             return rc;
         }
-        if (blocks > (long long)sms * 8) blocks = (long long)sms * 8;
-#define AVCTC_TOPK(NV, MODE)                                                                                        \
-    do {                                                                                                            \
-        static bool cfg = false;                                                                                    \
-        if (!cfg && pl.smem_topk > 48 * 1024) {                                                                     \
-            AVCTC_CUDA_RETURN(cudaFuncSetAttribute(beam_topk_kernel<NV, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                                   200 * 1024));                                                    \
-            cfg = true;                                                                                             \
-        }                                                                                                           \
-        beam_topk_kernel<NV, MODE><<<(unsigned)blocks, kTopkWarps * 32, pl.smem_topk, st>>>(bp);                    \
-    } while (0)
-#define AVCTC_TOPK_M(NV)                                                                                            \
-    do {                                                                                                            \
-        if (V == 32 * NV) AVCTC_TOPK(NV, 0);                                                                        \
-        else if (V > 32 * (NV - 1)) AVCTC_TOPK(NV, 1);                                                              \
-        else AVCTC_TOPK(NV, 2);                                                                                     \
-    } while (0)
-        if (need <= 4) AVCTC_TOPK(4, 2);
-        else if (need <= 8) AVCTC_TOPK(8, 2);
-        else if (need <= 16) AVCTC_TOPK(16, 2);
-        else if (need <= 25) AVCTC_TOPK_M(25);
-        else if (need <= 26) AVCTC_TOPK_M(26);
-        else AVCTC_TOPK_M(32);
-#undef AVCTC_TOPK_M
-#undef AVCTC_TOPK
-        AVCTC_CUDA_RETURN(cudaGetLastError());
+        const int rc_topk = topk_launch(bp, pl.smem_topk, sms, st);
+        if (rc_topk) return rc_topk;
         const size_t smem2 = pl.smem_recur_per_warp * kRecurWarps;
         static bool cfg2 = false;
         if (!cfg2 && smem2 > 48 * 1024) {

@@ -1,0 +1,96 @@
+"""CTC prefix beam search: ranked transcription hypotheses with their log-probabilities.
+
+    ctc_prefix_beam_search(log_probs[N,T,V], lengths=None, beam_width=5, nbest=1, blank=0) -> list[list[Hypothesis]]
+
+Unlike simple_beam_search, which keeps raw alignment paths and so returns the greedy collapse, the prefix beam search
+scores each prefix by the sum over all of its alignments and merges the alignments that collapse to the same text.
+The search is defined in DESIGN.md §4.13; the kernel (csrc/ctc_prefix_beam.cu) reproduces the CPU restatement in
+oracle/prefix_beam_oracle.py bit for bit, scores included.  Two kernel launches and one host sync per call.  CUDA
+tensors only.
+"""
+from __future__ import annotations
+
+from dataclasses import dataclass
+from typing import List
+
+import numpy as np
+import torch
+
+from . import _lib
+
+MAX_BEAM = 15
+
+
+@dataclass
+class Hypothesis:
+    """One decoded prefix: token ids (blanks and repeats already merged) and its natural-log probability."""
+    tokens: List[int]
+    score: float
+
+
+def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: int = 1,
+                           blank: int = 0) -> List[List[Hypothesis]]:
+    """log_probs: CUDA [N,T,V] log-probabilities (any float dtype; read as fp32).  lengths: frames to decode per
+    utterance (default T).  Returns, per utterance, up to nbest hypotheses, best first.  V <= 1024."""
+    _lib.require_cuda(log_probs, "log_probs")
+    if log_probs.dim() != 3:
+        raise RuntimeError("log_probs must be (N, T, V)")
+    N, T, V = log_probs.shape
+    B, nbest, blank = int(beam_width), int(nbest), int(blank)
+    if not 1 <= B <= MAX_BEAM:
+        raise ValueError(f"beam_width must be in [1, {MAX_BEAM}], got {B}")
+    if not 1 <= nbest <= B:
+        raise ValueError(f"nbest must be in [1, beam_width={B}], got {nbest}")
+    if not 0 <= blank < V:
+        raise ValueError(f"blank must be in [0, {V}), got {blank}")
+    lp = log_probs.detach()
+    if lp.dtype != torch.float32:
+        lp = lp.float()
+    if lp.stride(2) != 1:
+        lp = lp.contiguous()
+    dev = lp.device
+    L = _lib.lib()
+    ws_bytes = int(L.avctc_ctc_prefix_beam_workspace_bytes(N, T, V, B))
+    if ws_bytes == 0:
+        raise RuntimeError(f"ctc_prefix_beam_search: shape N={N}, T={T}, V={V} is not supported (V <= 1024)")
+    if lengths is not None:
+        lengths = torch.as_tensor(lengths).to(device=dev, dtype=torch.int64).contiguous()
+        if lengths.shape != (N,):
+            raise RuntimeError("lengths must be a 1-D tensor of one entry per utterance")
+    Tp = max(T, 1)
+    # every output in one device buffer, so that results and statuses come back with one copy
+    n_sc, n_len, n_st, n_tok = N * nbest * 8, N * nbest * 4, N * 4, N * nbest * Tp * 4
+    o_len = n_sc
+    o_st = o_len + n_len
+    o_tok = (o_st + n_st + 7) // 8 * 8
+    out = torch.empty(o_tok + n_tok, dtype=torch.uint8, device=dev)
+    scores = out[:o_len].view(torch.float64)
+    lens = out[o_len:o_st].view(torch.int32)
+    status = out[o_st:o_st + n_st].view(torch.int32)
+    tokens = out[o_tok:].view(torch.int32)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    with _lib.device_guard(dev):
+        _lib.check(L.avctc_ctc_prefix_beam(
+            lp.data_ptr(), lp.stride(0), lp.stride(1), N, T, V, lengths.data_ptr() if lengths is not None else None,
+            B, nbest, blank, tokens.data_ptr(), lens.data_ptr(), scores.data_ptr(), status.data_ptr(),
+            ws.data_ptr(), ws_bytes, _lib.stream_ptr(dev)), "avctc_ctc_prefix_beam")
+    host = out.cpu().numpy()                              # the one host sync
+    sc = host[:o_len].view(np.float64).reshape(N, nbest)
+    ln = host[o_len:o_st].view(np.int32).reshape(N, nbest)
+    st = host[o_st:o_st + n_st].view(np.int32)
+    tk = host[o_tok:].view(np.int32).reshape(N, nbest, Tp)
+    bad = np.flatnonzero(st)
+    if len(bad):
+        n = int(bad[0])
+        if st[n] == 1:
+            raise RuntimeError(f"ctc_prefix_beam_search: utterance {n}: log_probs contain NaN")
+        raise RuntimeError(f"ctc_prefix_beam_search: utterance {n}: length {int(lengths[n])} outside [0, {T}]")
+    res = []
+    for n in range(N):
+        row = []
+        for i in range(nbest):
+            if not sc[n, i] > -np.inf:                    # unused slot
+                break
+            row.append(Hypothesis(tk[n, i, :ln[n, i]].tolist(), float(sc[n, i])))
+        res.append(row)
+    return res

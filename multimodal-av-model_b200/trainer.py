@@ -33,6 +33,7 @@ from .beam_search import beam_search_batch, fast_decode
 from .contrastive import contrastive_loss_with_mask
 from .ctc import CTCLoss
 from .ddp import GradBucketReducer, broadcast_buffers, broadcast_module
+from .prefix_beam import ctc_prefix_beam_search
 
 
 def word_error_rate(refs, hyps):
@@ -148,9 +149,10 @@ class MultimodalTrainer:
         any_host = on_gpu and any(torch.is_tensor(v) and not v.is_cuda for v in batch.values())
         if not any_host:
             g = lambda k: batch[k].to(dev, non_blocking=True)
+            gt = lambda k: g(k) if k in batch else None          # transcripts: absent when only decoding
             lips = [g("lip1").permute(0, 2, 1, 3, 4).contiguous(), g("lip2").permute(0, 2, 1, 3, 4).contiguous()]
             return dict(lips=[(lambda t=t: t) for t in lips], audio=g("audio"), masks=[g("mask1"), g("mask2")],
-                        texts=[g("text1"), g("text2")], lens=[g("text1_lengths"), g("text2_lengths")])
+                        texts=[gt("text1"), gt("text2")], lens=[gt("text1_lengths"), gt("text2_lengths")])
         main = torch.cuda.current_stream(dev)
         if getattr(self, "_copy_stream", None) is None:
             self._copy_stream = torch.cuda.Stream(device=dev)
@@ -158,6 +160,8 @@ class MultimodalTrainer:
         out, events = {}, {}
         with torch.cuda.stream(cs):
             for k in ("audio", "mask1", "mask2", "text1", "text2", "text1_lengths", "text2_lengths"):
+                if k.startswith("text") and k not in batch:
+                    continue
                 out[k] = batch[k].to(dev, non_blocking=True)
             events["small"] = cs.record_event()
             for k in ("lip1", "lip2"):
@@ -173,7 +177,7 @@ class MultimodalTrainer:
                 return out[k]
             return get
         return dict(lips=[lip("lip1"), lip("lip2")], audio=out["audio"], masks=[out["mask1"], out["mask2"]],
-                    texts=[out["text1"], out["text2"]], lens=[out["text1_lengths"], out["text2_lengths"]])
+                    texts=[out.get("text1"), out.get("text2")], lens=[out.get("text1_lengths"), out.get("text2_lengths")])
 
     def _host_lengths(self, batch, key):
         """Utterance lengths (samples that are not padding, label 3) from the HOST copy of a mask, when there is one:
@@ -484,6 +488,33 @@ class MultimodalTrainer:
                                            end_sec=k[sp.end - 1] * self.hop_seconds + self.hop_seconds)
                             for sp in row])
             out.append(spk)
+        return out
+
+    # ------------------------------------------------------------------------------------------ transcription
+    def transcribe(self, batch, beam_width=None, nbest=1):
+        """What each speaker said: a CTC prefix beam search over the CTC head's log-probs, computed in eval mode with the
+        encoder -> fusion -> decoder1 path that align() uses, decoded on the fusion's input lengths.  The batch needs no
+        transcripts.  beam_width defaults to self.beam_width (at most 15).  Returns out[s][b] = [(text, score), ...],
+        best first, up to nbest per utterance; score is the hypothesis' natural-log probability."""
+        for m in (self.visual_encoder, self.audio_encoder, self.fusion_module, self.decoder1):
+            m.eval()
+        bw = self.beam_width if beam_width is None else beam_width
+        blank = self.tokenizer.blank_id
+        out = []
+        with torch.no_grad():
+            if hasattr(self.audio_encoder, "begin_step"):
+                self.audio_encoder.begin_step()
+            d = self._to_dev(batch)
+            with torch.autocast("cuda", dtype=self.autocast_dtype, enabled=str(self.device).startswith("cuda")):
+                for s in range(2):
+                    vis = self.visual_encoder(d["lips"][s]())
+                    aud, _ = self.audio_encoder(d["audio"], attention_mask=(d["masks"][s] != 3))
+                    t_enc = aud.shape[1]
+                    mask_ds = F.interpolate(d["masks"][s].unsqueeze(1).float(), size=t_enc, mode="nearest").squeeze(1).long()
+                    fused, il = self.fusion_module(vis, aud, mask_ds)
+                    lp = self.decoder1(fused)
+                    hyps = ctc_prefix_beam_search(lp, il, beam_width=bw, nbest=nbest, blank=blank)
+                    out.append([[(fast_decode(h.tokens, self.tokenizer), h.score) for h in row] for row in hyps])
         return out
 
     def _piece(self, token):
