@@ -186,6 +186,36 @@ AVCTC_API int avctc_ctc_prefix_beam(const float* log_probs, int64_t stride_n, in
                                     size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * The same search with shallow fusion of a token-level back-off n-gram LM (DESIGN.md §4.14, restated in
+ * oracle/prefix_beam_lm_oracle.py, whose results it reproduces bit for bit).  Each prefix carries an LM score L
+ * (fp64 natural log): an extension s+c adds lm_weight * ln P(c | <s> s) + token_bonus, and candidates are ranked by
+ * acoustic + L.  After the last frame lm_weight * ln P(</s> | <s> s) is added and the beam re-ranked.
+ * LM words have ids 0..num_words-1 (num_words <= 2048, 11 bits).  An n-gram w1..wn is the key
+ * sum_i w_i << 11*(n-i); the order-n table (n = 2..5) is table[n-2], `capacity` 16-byte entries {uint64 key; float
+ * log10 p; float log10 back-off}, empty slots keyed ~0, at most half full, probed linearly from
+ * slot = h & (capacity-1), h = key * 0x9E3779B97F4A7C15 (mod 2^64), h ^= h >> 29.  Unigrams are dense.
+ * `lm` is a HOST pointer to the descriptor (read during the call); the pointers inside it are device memory.
+ * lm_weight finite and >= 0, token_bonus finite, order 1..5, map_len == V; AVCTC_ERR_BAD_ARG otherwise, before any
+ * launch.  Outputs as avctc_ctc_prefix_beam, with out_scores = out_acoustic + out_lm per hypothesis (unused slots
+ * -inf in all three).  Same workspace query, two kernel launches, no host sync.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct avctc_ngram_lm {
+    int order;                   /* 1..5 */
+    int num_words;               /* LM word ids are 0..num_words-1, num_words <= 2048 */
+    int bos, eos;                /* word ids of <s> and </s> */
+    int map_len;                 /* entries of token_word: must equal V */
+    const int32_t* token_word;   /* device [map_len]: model token -> LM word id (<unk>'s id for a piece the LM lacks) */
+    const float* unigram;        /* device [num_words][2]: log10 p, log10 back-off (0 when absent) */
+    const void* table[4];        /* device tables of orders 2..5 (unused past `order`) */
+    uint64_t capacity[4];        /* entries of each table: a power of two >= 2 */
+} avctc_ngram_lm;
+AVCTC_API int avctc_ctc_prefix_beam_lm(const float* log_probs, int64_t stride_n, int64_t stride_t, int N, int T, int V,
+                                       const int64_t* lengths, int beam, int nbest, int blank, const avctc_ngram_lm* lm,
+                                       double lm_weight, double token_bonus, int32_t* out_tokens, int32_t* out_len,
+                                       double* out_scores, double* out_acoustic, double* out_lm, int32_t* status,
+                                       void* workspace, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Fusion path dense contraction (tcgen05 + TMEM + TMA) — replaces the cuBLAS GEMMs under
  *   nn.Linear x4            /root/reference/model/fusion_module.py:57,58,63; model/decoder.py:24
  *   nn.MultiheadAttention   /root/reference/model/fusion_module.py:61 (in/out projections, Q.K^T, P.V)

@@ -1,15 +1,22 @@
 """CTC prefix beam search: ranked transcription hypotheses with their log-probabilities.
 
-    ctc_prefix_beam_search(log_probs[N,T,V], lengths=None, beam_width=5, nbest=1, blank=0) -> list[list[Hypothesis]]
+    ctc_prefix_beam_search(log_probs[N,T,V], lengths=None, beam_width=5, nbest=1, blank=0,
+                           lm=None, lm_weight=0.5, token_bonus=0.0) -> list[list[Hypothesis]]
 
 Unlike simple_beam_search, which keeps raw alignment paths and so returns the greedy collapse, the prefix beam search
 scores each prefix by the sum over all of its alignments and merges the alignments that collapse to the same text.
 The search is defined in DESIGN.md §4.13; the kernel (csrc/ctc_prefix_beam.cu) reproduces the CPU restatement in
 oracle/prefix_beam_oracle.py bit for bit, scores included.  Two kernel launches and one host sync per call.  CUDA
 tensors only.
+
+With an n-gram LM (ngram_lm.NgramLM), the search fuses it shallowly (DESIGN.md §4.14, oracle/prefix_beam_lm_oracle.py):
+prefixes are ranked by acoustic + lm_weight * ln P_LM + token_bonus * length, </s> included at the end, and each
+hypothesis is an LMHypothesis carrying both parts.
 """
 from __future__ import annotations
 
+import ctypes
+import math
 from dataclasses import dataclass
 from typing import List
 
@@ -17,6 +24,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .ngram_lm import NgramLM
 
 MAX_BEAM = 15
 
@@ -28,10 +36,20 @@ class Hypothesis:
     score: float
 
 
-def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: int = 1,
-                           blank: int = 0) -> List[List[Hypothesis]]:
+@dataclass
+class LMHypothesis(Hypothesis):
+    """A hypothesis of the LM-fused search: score = acoustic_score + lm_score (one fp64 add), where acoustic_score is
+    the CTC log-probability and lm_score = lm_weight * ln P_LM(tokens </s>) + token_bonus * len(tokens)."""
+    acoustic_score: float
+    lm_score: float
+
+
+def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: int = 1, blank: int = 0,
+                           lm: NgramLM = None, lm_weight: float = 0.5, token_bonus: float = 0.0) -> List[List[Hypothesis]]:
     """log_probs: CUDA [N,T,V] log-probabilities (any float dtype; read as fp32).  lengths: frames to decode per
-    utterance (default T).  Returns, per utterance, up to nbest hypotheses, best first.  V <= 1024."""
+    utterance (default T).  Returns, per utterance, up to nbest hypotheses, best first.  V <= 1024.  With `lm`, an
+    NgramLM built for this model's V pieces, hypotheses are LMHypothesis ranked by the fused score; lm_weight must be
+    finite and >= 0, token_bonus finite."""
     _lib.require_cuda(log_probs, "log_probs")
     if log_probs.dim() != 3:
         raise RuntimeError("log_probs must be (N, T, V)")
@@ -43,6 +61,16 @@ def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: 
         raise ValueError(f"nbest must be in [1, beam_width={B}], got {nbest}")
     if not 0 <= blank < V:
         raise ValueError(f"blank must be in [0, {V}), got {blank}")
+    if lm is not None:
+        if not isinstance(lm, NgramLM):
+            raise TypeError(f"lm must be an NgramLM, got {type(lm).__name__}")
+        if lm.vocab_size != V:
+            raise ValueError(f"the LM was built for {lm.vocab_size} pieces, log_probs have V={V} classes")
+        alpha, beta = float(lm_weight), float(token_bonus)
+        if not (math.isfinite(alpha) and alpha >= 0.0):
+            raise ValueError(f"lm_weight must be finite and >= 0, got {lm_weight}")
+        if not math.isfinite(beta):
+            raise ValueError(f"token_bonus must be finite, got {token_bonus}")
     lp = log_probs.detach()
     if lp.dtype != torch.float32:
         lp = lp.float()
@@ -58,8 +86,10 @@ def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: 
         if lengths.shape != (N,):
             raise RuntimeError("lengths must be a 1-D tensor of one entry per utterance")
     Tp = max(T, 1)
-    # every output in one device buffer, so that results and statuses come back with one copy
-    n_sc, n_len, n_st, n_tok = N * nbest * 8, N * nbest * 4, N * 4, N * nbest * Tp * 4
+    # every output in one device buffer, so that results and statuses come back with one copy; with an LM the scores
+    # are [3][N][nbest]: fused, acoustic, LM
+    nsc = 1 if lm is None else 3
+    n_sc, n_len, n_st, n_tok = nsc * N * nbest * 8, N * nbest * 4, N * 4, N * nbest * Tp * 4
     o_len = n_sc
     o_st = o_len + n_len
     o_tok = (o_st + n_st + 7) // 8 * 8
@@ -70,12 +100,22 @@ def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: 
     tokens = out[o_tok:].view(torch.int32)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
     with _lib.device_guard(dev):
-        _lib.check(L.avctc_ctc_prefix_beam(
-            lp.data_ptr(), lp.stride(0), lp.stride(1), N, T, V, lengths.data_ptr() if lengths is not None else None,
-            B, nbest, blank, tokens.data_ptr(), lens.data_ptr(), scores.data_ptr(), status.data_ptr(),
-            ws.data_ptr(), ws_bytes, _lib.stream_ptr(dev)), "avctc_ctc_prefix_beam")
+        if lm is None:
+            _lib.check(L.avctc_ctc_prefix_beam(
+                lp.data_ptr(), lp.stride(0), lp.stride(1), N, T, V, lengths.data_ptr() if lengths is not None else None,
+                B, nbest, blank, tokens.data_ptr(), lens.data_ptr(), scores.data_ptr(), status.data_ptr(),
+                ws.data_ptr(), ws_bytes, _lib.stream_ptr(dev)), "avctc_ctc_prefix_beam")
+        else:
+            desc = lm.descriptor(dev)
+            sc3 = scores.view(3, N * nbest)
+            _lib.check(L.avctc_ctc_prefix_beam_lm(
+                lp.data_ptr(), lp.stride(0), lp.stride(1), N, T, V, lengths.data_ptr() if lengths is not None else None,
+                B, nbest, blank, ctypes.addressof(desc), alpha, beta, tokens.data_ptr(), lens.data_ptr(),
+                sc3[0].data_ptr(), sc3[1].data_ptr(), sc3[2].data_ptr(), status.data_ptr(), ws.data_ptr(), ws_bytes,
+                _lib.stream_ptr(dev)), "avctc_ctc_prefix_beam_lm")
     host = out.cpu().numpy()                              # the one host sync
-    sc = host[:o_len].view(np.float64).reshape(N, nbest)
+    sc_all = host[:o_len].view(np.float64).reshape(nsc, N, nbest)
+    sc = sc_all[0]
     ln = host[o_len:o_st].view(np.int32).reshape(N, nbest)
     st = host[o_st:o_st + n_st].view(np.int32)
     tk = host[o_tok:].view(np.int32).reshape(N, nbest, Tp)
@@ -91,6 +131,10 @@ def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: 
         for i in range(nbest):
             if not sc[n, i] > -np.inf:                    # unused slot
                 break
-            row.append(Hypothesis(tk[n, i, :ln[n, i]].tolist(), float(sc[n, i])))
+            if lm is None:
+                row.append(Hypothesis(tk[n, i, :ln[n, i]].tolist(), float(sc[n, i])))
+            else:
+                row.append(LMHypothesis(tk[n, i, :ln[n, i]].tolist(), float(sc[n, i]), float(sc_all[1, n, i]),
+                                        float(sc_all[2, n, i])))
         res.append(row)
     return res

@@ -491,11 +491,12 @@ class MultimodalTrainer:
         return out
 
     # ------------------------------------------------------------------------------------------ transcription
-    def transcribe(self, batch, beam_width=None, nbest=1):
+    def transcribe(self, batch, beam_width=None, nbest=1, lm=None, lm_weight=0.5, token_bonus=0.0):
         """What each speaker said: a CTC prefix beam search over the CTC head's log-probs, computed in eval mode with the
         encoder -> fusion -> decoder1 path that align() uses, decoded on the fusion's input lengths.  The batch needs no
         transcripts.  beam_width defaults to self.beam_width (at most 15).  Returns out[s][b] = [(text, score), ...],
-        best first, up to nbest per utterance; score is the hypothesis' natural-log probability."""
+        best first, up to nbest per utterance; score is the hypothesis' natural-log probability, or with `lm` (an
+        NgramLM over this tokenizer's pieces) the fused score acoustic + lm_weight * ln P_LM + token_bonus * length."""
         for m in (self.visual_encoder, self.audio_encoder, self.fusion_module, self.decoder1):
             m.eval()
         bw = self.beam_width if beam_width is None else beam_width
@@ -513,7 +514,8 @@ class MultimodalTrainer:
                     mask_ds = F.interpolate(d["masks"][s].unsqueeze(1).float(), size=t_enc, mode="nearest").squeeze(1).long()
                     fused, il = self.fusion_module(vis, aud, mask_ds)
                     lp = self.decoder1(fused)
-                    hyps = ctc_prefix_beam_search(lp, il, beam_width=bw, nbest=nbest, blank=blank)
+                    hyps = ctc_prefix_beam_search(lp, il, beam_width=bw, nbest=nbest, blank=blank, lm=lm,
+                                                  lm_weight=lm_weight, token_bonus=token_bonus)
                     out.append([[(fast_decode(h.tokens, self.tokenizer), h.score) for h in row] for row in hyps])
         return out
 
