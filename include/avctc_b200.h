@@ -216,6 +216,39 @@ AVCTC_API int avctc_ctc_prefix_beam_lm(const float* log_probs, int64_t stride_n,
                                        void* workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * The same search with contextual biasing towards a phrase list, with or without the n-gram LM (DESIGN.md §4.15,
+ * restated in oracle/context_graph_oracle.py, whose results it reproduces bit for bit).  The phrases form an
+ * Aho-Corasick automaton: node 0 is the root, node v has the depth potential phi(v) (the sum of its path's per-token
+ * weights) and the completion credit omega(v) (phi of the first node on v's fail chain that ends a phrase, else 0).
+ * Each prefix carries a node u and a bias score G (root and 0 for the empty prefix): an extension s+c moves to
+ * v = delta(u, c) and adds (phi(v) - phi(u)) + omega(v) to G; candidates are ranked by (acoustic + L) + G, or
+ * acoustic + G without an LM.  After the last frame bias = G - phi(u) and score = (acoustic + lm) + bias.
+ * Candidates still come from the acoustic top-(2B+1) list of each frame: a phrase token outside it cannot be boosted.
+ * Tables (device memory, `ctx` a HOST pointer read during the call): token_sym[map_len] maps a model token to its
+ * context-alphabet symbol 0..alphabet-1, or -1 for a token of no phrase (which always returns to the root);
+ * delta[num_nodes * alphabet] is the dense transition table, row-major by node; node[num_nodes] = (phi, omega).
+ * `lm` NULL = no LM (lm_weight and token_bonus are ignored; out_lm gets 0 per hypothesis), else it is checked as by
+ * avctc_ctc_prefix_beam_lm.  ctx non-NULL with num_nodes >= 1, map_len == V and alphabet in 1..V; AVCTC_ERR_BAD_ARG
+ * otherwise, before any launch.  Outputs as avctc_ctc_prefix_beam_lm plus out_bias, with out_scores =
+ * (out_acoustic + out_lm) + out_bias per hypothesis (unused slots -inf in all four).  Same workspace query, two
+ * kernel launches, no host sync.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct avctc_context_graph {
+    int num_nodes;               /* automaton nodes, root = 0 */
+    int alphabet;                /* distinct phrase tokens: 1..V */
+    const int32_t* token_sym;    /* device [map_len]: model token -> symbol, -1 when no phrase uses the token */
+    int map_len;                 /* entries of token_sym: must equal V */
+    const int32_t* delta;        /* device [num_nodes][alphabet]: next node */
+    const double* node;          /* device [num_nodes][2]: phi, omega (16-byte aligned) */
+} avctc_context_graph;
+AVCTC_API int avctc_ctc_prefix_beam_biased(const float* log_probs, int64_t stride_n, int64_t stride_t, int N, int T,
+                                           int V, const int64_t* lengths, int beam, int nbest, int blank,
+                                           const avctc_ngram_lm* lm, double lm_weight, double token_bonus,
+                                           const avctc_context_graph* ctx, int32_t* out_tokens, int32_t* out_len,
+                                           double* out_scores, double* out_acoustic, double* out_lm, double* out_bias,
+                                           int32_t* status, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Fusion path dense contraction (tcgen05 + TMEM + TMA) — replaces the cuBLAS GEMMs under
  *   nn.Linear x4            /root/reference/model/fusion_module.py:57,58,63; model/decoder.py:24
  *   nn.MultiheadAttention   /root/reference/model/fusion_module.py:61 (in/out projections, Q.K^T, P.V)

@@ -12,6 +12,7 @@ hyphen).  Public names mirror the reference modules (SURVEY.md §8b):
     forced_align, merge_tokens, TokenSpan     torchaudio.functional's CTC forced alignment, batched (align.py)
     ctc_prefix_beam_search, Hypothesis        CTC prefix beam search with N-best hypotheses and scores (prefix_beam.py)
     NgramLM, LMHypothesis                     token n-gram LM shallow fusion for that search (ngram_lm.py)
+    ContextGraph, BiasedHypothesis            contextual biasing towards a phrase list in that search (context_graph.py)
 """
 from . import _lib
 from .ctc import CTCLoss, ctc_loss
@@ -32,7 +33,8 @@ _optional("fusion_module", ["CrossAttentionFusion"])
 _optional("decoder", ["CTCDecoder"])
 _optional("contrastive", ["contrastive_loss_with_mask"])
 _optional("align", ["forced_align", "merge_tokens", "merge_tokens_batch", "TokenSpan"])
-_optional("prefix_beam", ["ctc_prefix_beam_search", "Hypothesis", "LMHypothesis"])
+_optional("prefix_beam", ["ctc_prefix_beam_search", "Hypothesis", "LMHypothesis", "BiasedHypothesis"])
 _optional("ngram_lm", ["NgramLM"])
+_optional("context_graph", ["ContextGraph"])
 _optional("trainer", ["MultimodalTrainer"])
 _optional("encoders", ["VisualEncoder", "AudioEncoder"])

@@ -42,6 +42,8 @@ SIGNATURES = {
     "avctc_ctc_prefix_beam": (_i, [_vp, _i64, _i64, _i, _i, _i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "avctc_ctc_prefix_beam_lm": (_i, [_vp, _i64, _i64, _i, _i, _i, _vp, _i, _i, _i, _vp, _d, _d, _vp, _vp, _vp, _vp,
                                       _vp, _vp, _vp, _sz, _vp]),
+    "avctc_ctc_prefix_beam_biased": (_i, [_vp, _i64, _i64, _i, _i, _i, _vp, _i, _i, _i, _vp, _d, _d, _vp, _vp, _vp,
+                                          _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "avctc_gemm_bf16": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _vp, _i, ctypes.c_longlong, ctypes.c_longlong,
                              ctypes.c_longlong, _vp, _i, ctypes.c_float, _i, _vp]),
     "avctc_resample_workspace_bytes": (_sz, [_i, _i]),
@@ -105,10 +107,16 @@ class NgramLMDesc(ctypes.Structure):
                 ("capacity", ctypes.c_uint64 * 4)]
 
 
+class ContextGraphDesc(ctypes.Structure):
+    """Mirror of avctc_context_graph (include/avctc_b200.h)."""
+    _fields_ = [("num_nodes", _i), ("alphabet", _i), ("token_sym", ctypes.c_void_p), ("map_len", _i),
+                ("delta", ctypes.c_void_p), ("node", ctypes.c_void_p)]
+
+
 # kernels launched by each entry point (bench.py reports "gpu_launches" from this table); CTC forward / backward with a
 # workspace = the probability-domain kernel + its guarded log-domain twin (which exits at once unless the range guard tripped)
 KERNELS = {"avctc_ctc_forward": 2, "avctc_ctc_reduce": 1, "avctc_ctc_backward": 2, "avctc_ctc_forward_backward": 5, "avctc_ctc_scale_grad": 1, "avctc_ctc_align": 1, "avctc_beam_search": 2,
-           "avctc_ctc_prefix_beam": 2, "avctc_ctc_prefix_beam_lm": 2,
+           "avctc_ctc_prefix_beam": 2, "avctc_ctc_prefix_beam_lm": 2, "avctc_ctc_prefix_beam_biased": 2,
            "avctc_gemm_bf16": 1, "avctc_resample_forward": 2, "avctc_resample_backward": 1, "avctc_softmax_forward": 1,
            "avctc_softmax_backward": 1, "avctc_colsum": 1, "avctc_log_softmax_forward": 1,
            "avctc_log_softmax_backward": 1, "avctc_infonce_forward": 4, "avctc_infonce_backward": 2,

@@ -11,7 +11,8 @@
 // Prefixes are trie nodes (parent << 10 | token) in shared memory, or in the workspace when 1 + T*B of them do not fit.
 // A prefix that left the beam and comes back gets a new node, so two nodes can hold the same prefix: identity is
 // decided by content, walking both parent chains until the nodes meet (never by a hash).
-// ctc_prefix_beam_lm_kernel (below) is the same recurrence with shallow fusion of a token n-gram LM (DESIGN.md §4.14).
+// ctc_prefix_beam_lm_kernel (below) is the same recurrence with shallow fusion of a token n-gram LM (DESIGN.md §4.14)
+// and / or contextual biasing towards a phrase list (§4.15).
 #include <cmath>
 
 #include "common.cuh"
@@ -291,9 +292,26 @@ __device__ __forceinline__ double lm10(const PbLm& lm, unsigned long long hist, 
     return __dadd_rn(acc, (double)__ldg(lm.unigram + w).x);
 }
 
+// Contextual biasing (DESIGN.md §4.15; oracle/context_graph_oracle.py): each entry also carries its node u in the
+// phrase automaton and an fp64 bias score G.  An extension s+c moves to v = delta(u, c) and adds
+// (phi(v) - phi(u)) + omega(v); the key gains + G'.  After the last frame G - phi(u) withdraws an unfinished match.
+struct PbCtx {
+    const int32_t* token_sym;              // [V]: context-alphabet symbol of a token, -1 = not in any phrase
+    const int32_t* delta;                  // [num_nodes][alphabet]
+    const double2* node;                   // [num_nodes]: (phi, omega)
+    int alphabet;
+};
+
+// Per-warp shared memory of the biased instances: kPbLmFixedBytes, then cG[kPbCand], nx_G[16], cctx[kPbCand], nx_ctx[16].
+constexpr int kPbBiasFixedBytes = kPbLmFixedBytes + kPbCand * (8 + 4) + 16 * (8 + 4);
+
+// kLm: n-gram fusion (§4.14); kBias: contextual biasing (§4.15).  <true, false> is the LM search of §4.14; its
+// parameters come first so that the instance compiles to the same code as before the biasing was added.
+template <bool kLm, bool kBias>
 __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const PbParams p, const PbLm lm,
                                                                           double* out_ac, double* out_lm,
-                                                                          const int per_warp_bytes) {
+                                                                          const int per_warp_bytes, const PbCtx cx,
+                                                                          double* out_bias) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int n = blockIdx.x * kPbWarps + warp;
@@ -307,17 +325,25 @@ __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const
     double* nx_L = nx_tot + 16;
     int* nx_src = reinterpret_cast<int*>(nx_L + 16);
     int* nx_tok = nx_src + 16;
+    double* cG = reinterpret_cast<double*>(nx_tok + 16);             // candidate G' and context node (biasing only)
+    double* nx_G = cG + kPbCand;
+    int* cctx = reinterpret_cast<int*>(nx_G + 16);
+    int* nx_ctx = cctx + kPbCand;
     volatile uint32_t* nodes = p.nodes_g ? p.nodes_g + (size_t)n * p.node_cap
-                                         : reinterpret_cast<uint32_t*>(mine + kPbLmFixedBytes);
+                                         : reinterpret_cast<uint32_t*>(mine + (kBias ? kPbBiasFixedBytes : kPbLmFixedBytes));
     const int B = p.beam, S = B + 1, k = p.k, blank = p.blank;
     const size_t o0 = (size_t)n * p.nbest;
     int32_t* olen = p.out_len + o0;
     double* osc = p.out_scores + o0;
     double* oac = out_ac + o0;
     double* olm = out_lm + o0;
+    double* obias = kBias ? out_bias + o0 : nullptr;
     const long long fl = p.lengths ? p.lengths[n] : p.T;
     if (fl < 0 || fl > p.T) {
-        if (lane < p.nbest) { olen[lane] = 0; osc[lane] = kNegInfD; oac[lane] = kNegInfD; olm[lane] = kNegInfD; }
+        if (lane < p.nbest) {
+            olen[lane] = 0; osc[lane] = kNegInfD; oac[lane] = kNegInfD; olm[lane] = kNegInfD;
+            if constexpr (kBias) obias[lane] = kNegInfD;
+        }
         if (lane == 0) p.status[n] = 2;
         return;
     }
@@ -334,19 +360,26 @@ __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const
     int last = -1, len = 0, node = 0, nb = 1, next_node = 1, st = 0;
     unsigned long long hist = hmax > 0 ? (unsigned long long)lm.bos : 0ull;
     int hlen = hmax > 0 ? 1 : 0;
+    double G = 0.0, phi = 0.0;                 // bias score and phi of the entry's context node ctx (root: 0)
+    int ctx = 0;
     float kv = 0.f, lpb = 0.f, lpl = 0.f;      // this frame's K_t entry (lane j), lp[t,blank], lp[t,last]
-    int ki = -1, kw = 0;                       // its class and LM word
+    int ki = -1, kw = 0, ks = -1;              // its class, LM word and context symbol
     if (frames > 0) {
-        if (lane < k) { kv = tkv[lane]; ki = tki[lane]; kw = ki >= 0 && ki < p.V ? lm.token_word[ki] : 0; }
+        if (lane < k) {
+            kv = tkv[lane]; ki = tki[lane];
+            if constexpr (kLm) kw = ki >= 0 && ki < p.V ? lm.token_word[ki] : 0;
+            if constexpr (kBias) ks = ki >= 0 && ki < p.V ? __ldg(cx.token_sym + ki) : -1;
+        }
         lpb = base[blank];
     }
     for (int t = 0; t < frames; ++t) {
         const float kv_t = kv, lpb_t = lpb, lpl_t = lpl;
-        const int ki_t = ki, kw_t = kw;
+        const int ki_t = ki, kw_t = kw, ks_t = ks;
         if (t + 1 < frames && lane < k) {
             kv = tkv[(size_t)(t + 1) * k + lane];
             ki = tki[(size_t)(t + 1) * k + lane];
-            kw = ki >= 0 && ki < p.V ? lm.token_word[ki] : 0;
+            if constexpr (kLm) kw = ki >= 0 && ki < p.V ? lm.token_word[ki] : 0;
+            if constexpr (kBias) ks = ki >= 0 && ki < p.V ? __ldg(cx.token_sym + ki) : -1;
         }
         const float k0 = __shfl_sync(kFullMask, kv_t, 0);
         if (k0 != k0) { st = 1; break; }
@@ -373,8 +406,14 @@ __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const
             const double stot = log_add(spb, spnb);
             const bool ok = stot > kNegInfD;
             ctot[lane * S] = ok ? stot : kNegInfD;
-            ckey[lane * S] = ok ? __dadd_rn(stot, L) : nan;
-            cL[lane * S] = L;
+            if constexpr (kBias) {
+                ckey[lane * S] = ok ? __dadd_rn(kLm ? __dadd_rn(stot, L) : stot, G) : nan;
+                cG[lane * S] = G;
+                cctx[lane * S] = ctx;
+            } else {
+                ckey[lane * S] = ok ? __dadd_rn(stot, L) : nan;
+            }
+            if constexpr (kLm) cL[lane * S] = L;
             ctok[lane * S] = -1;
         }
         unsigned inbeam = 0;
@@ -387,16 +426,33 @@ __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const
         // slots s*S + 1 .. s*S + B
         for (int s = 0; s < nb; ++s) {
             const double s_tot = __shfl_sync(kFullMask, tot, s), s_pb = __shfl_sync(kFullMask, pb, s);
-            const double s_L = __shfl_sync(kFullMask, L, s);
-            const unsigned long long s_hist = __shfl_sync(kFullMask, hist, s);
-            const int s_last = __shfl_sync(kFullMask, last, s), s_hlen = __shfl_sync(kFullMask, hlen, s);
+            const double s_L = kLm ? __shfl_sync(kFullMask, L, s) : 0.0;
+            const unsigned long long s_hist = kLm ? __shfl_sync(kFullMask, hist, s) : 0ull;
+            const int s_last = __shfl_sync(kFullMask, last, s), s_hlen = kLm ? __shfl_sync(kFullMask, hlen, s) : 0;
             const double e = __dadd_rn(ki_t == s_last ? s_pb : s_tot, (double)kv_t);
             const bool ok = tok_ok && !((inbeam >> s) & 1u) && e > kNegInfD;
             double Lc = 0.0, key = 0.0;
             if (ok) {
-                const double d = __dadd_rn(__dmul_rn(lm.alpha, __dmul_rn(lm10(lm, s_hist, s_hlen, kw_t), kLn10)), lm.beta);
-                Lc = __dadd_rn(s_L, d);
-                key = __dadd_rn(e, Lc);
+                if constexpr (kLm) {
+                    const double d = __dadd_rn(__dmul_rn(lm.alpha, __dmul_rn(lm10(lm, s_hist, s_hlen, kw_t), kLn10)), lm.beta);
+                    Lc = __dadd_rn(s_L, d);
+                    key = __dadd_rn(e, Lc);
+                } else {
+                    key = e;
+                }
+            }
+            double Gc = 0.0;
+            int vc = 0;
+            if constexpr (kBias) {
+                // v = delta(u_s, c): a token outside every phrase returns to the root
+                const double s_G = __shfl_sync(kFullMask, G, s), s_phi = __shfl_sync(kFullMask, phi, s);
+                const int s_ctx = __shfl_sync(kFullMask, ctx, s);
+                if (ok) {
+                    vc = ks_t < 0 ? 0 : __ldg(cx.delta + (size_t)s_ctx * cx.alphabet + ks_t);
+                    const double2 nv = __ldg(cx.node + vc);
+                    Gc = __dadd_rn(s_G, __dadd_rn(__dsub_rn(nv.x, s_phi), nv.y));
+                    key = __dadd_rn(key, Gc);
+                }
             }
             const unsigned m = __ballot_sync(kFullMask, ok);
             int r = 0;
@@ -408,7 +464,8 @@ __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const
             if (ok && r < B) {
                 ckey[slot0 + r] = key;
                 ctot[slot0 + r] = e;
-                cL[slot0 + r] = Lc;
+                if constexpr (kLm) cL[slot0 + r] = Lc;
+                if constexpr (kBias) { cG[slot0 + r] = Gc; cctx[slot0 + r] = vc; }
                 ctok[slot0 + r] = ki_t;
             }
             const int cnt = min(__popc(m), B);
@@ -427,7 +484,12 @@ __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const
                     const double o = ckey[q];
                     r += (o > v) || (o == v && q < m);
                 }
-                if (r < B) { nx_tot[r] = ctot[m]; nx_L[r] = cL[m]; nx_src[r] = m / S; nx_tok[r] = ctok[m]; }
+                if (r < B) {
+                    nx_tot[r] = ctot[m];
+                    if constexpr (kLm) nx_L[r] = cL[m];
+                    if constexpr (kBias) { nx_G[r] = cG[m]; nx_ctx[r] = cctx[m]; }
+                    nx_src[r] = m / S; nx_tok[r] = ctok[m];
+                }
             }
         }
         const int nb_new = min(B, (int)__reduce_add_sync(kFullMask, (unsigned)valid));
@@ -436,19 +498,21 @@ __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const
         const int src = live ? nx_src[lane] : 0;
         const int tok = live ? nx_tok[lane] : -1;
         const double ntot = live ? nx_tot[lane] : kNegInfD;
-        const double nL = live ? nx_L[lane] : 0.0;
+        const double nL = kLm && live ? nx_L[lane] : 0.0;
         const double o_spb = __shfl_sync(kFullMask, spb, src), o_spnb = __shfl_sync(kFullMask, spnb, src);
         const int o_last = __shfl_sync(kFullMask, last, src), o_len = __shfl_sync(kFullMask, len, src);
-        const int o_node = __shfl_sync(kFullMask, node, src), o_hlen = __shfl_sync(kFullMask, hlen, src);
-        const unsigned long long o_hist = __shfl_sync(kFullMask, hist, src);
+        const int o_node = __shfl_sync(kFullMask, node, src), o_hlen = kLm ? __shfl_sync(kFullMask, hlen, src) : 0;
+        const unsigned long long o_hist = kLm ? __shfl_sync(kFullMask, hist, src) : 0ull;
         const bool is_ext = live && tok >= 0;
         const unsigned em = __ballot_sync(kFullMask, is_ext);
         if (is_ext) {
             const int id = next_node + __popc(em & lt);
             nodes[id] = ((uint32_t)o_node << 10) | (uint32_t)tok;
             pb = kNegInfD; pnb = ntot; last = tok; len = o_len + 1; node = id;
-            hist = ((o_hist << 11) | (unsigned)lm.token_word[tok]) & hmask;
-            hlen = min(o_hlen + 1, hmax);
+            if constexpr (kLm) {
+                hist = ((o_hist << 11) | (unsigned)lm.token_word[tok]) & hmask;
+                hlen = min(o_hlen + 1, hmax);
+            }
         } else if (live) {
             pb = o_spb; pnb = o_spnb; last = o_last; len = o_len; node = o_node;
             hist = o_hist; hlen = o_hlen;
@@ -458,6 +522,11 @@ __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const
         }
         tot = ntot;
         L = nL;
+        if constexpr (kBias) {
+            G = live ? nx_G[lane] : 0.0;
+            ctx = live ? nx_ctx[lane] : 0;
+            phi = live ? __ldg(&cx.node[ctx].x) : 0.0;
+        }
         next_node += __popc(em);
         nb = nb_new;
         __syncwarp();
@@ -467,12 +536,22 @@ __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const
             if (live && len > 0) lpl = row[last];
         }
     }
-    // end of sentence: E = alpha * ln P(</s> | history), then a stable re-rank by tot + (L + E)
+    // end of sentence: E = alpha * ln P(</s> | history) (0 without an LM) and bias = G - phi(u), then a stable
+    // re-rank by (tot + (L + E)) + bias
     const bool have = st == 0 && lane < nb;
-    double lms = kNegInfD, fin = kNegInfD;
+    double lms = kNegInfD, fin = kNegInfD, bias = kNegInfD;
     if (have) {
-        lms = __dadd_rn(L, __dmul_rn(lm.alpha, __dmul_rn(lm10(lm, hist, hlen, lm.eos), kLn10)));
-        fin = __dadd_rn(tot, lms);
+        if constexpr (kLm) {
+            lms = __dadd_rn(L, __dmul_rn(lm.alpha, __dmul_rn(lm10(lm, hist, hlen, lm.eos), kLn10)));
+            fin = __dadd_rn(tot, lms);
+        } else {
+            lms = 0.0;
+            fin = __dadd_rn(tot, lms);
+        }
+        if constexpr (kBias) {
+            bias = __dsub_rn(G, phi);
+            fin = __dadd_rn(fin, bias);
+        }
     }
     int r = 0;
     for (int j = 0; j < nb; ++j) {
@@ -481,6 +560,7 @@ __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const
     }
     if (have && r < p.nbest) {
         olen[r] = len; osc[r] = fin; oac[r] = tot; olm[r] = lms;
+        if constexpr (kBias) obias[r] = bias;
         int32_t* dst = p.out_tokens + (o0 + r) * p.T;
         int x = node;
         for (int j = len - 1; j >= 0; --j) {
@@ -490,7 +570,10 @@ __global__ void __launch_bounds__(kPbWarps * 32) ctc_prefix_beam_lm_kernel(const
         }
     }
     const int used = st == 0 ? min(nb, p.nbest) : 0;
-    if (lane >= used && lane < p.nbest) { olen[lane] = 0; osc[lane] = kNegInfD; oac[lane] = kNegInfD; olm[lane] = kNegInfD; }
+    if (lane >= used && lane < p.nbest) {
+        olen[lane] = 0; osc[lane] = kNegInfD; oac[lane] = kNegInfD; olm[lane] = kNegInfD;
+        if constexpr (kBias) obias[lane] = kNegInfD;
+    }
     if (lane == 0) p.status[n] = st;
 }
 
@@ -567,25 +650,33 @@ extern "C" int avctc_ctc_prefix_beam(const float* log_probs, int64_t stride_n, i
     return (int)cudaGetLastError();
 }
 
-extern "C" int avctc_ctc_prefix_beam_lm(const float* log_probs, int64_t stride_n, int64_t stride_t, int N, int T, int V,
-                                        const int64_t* lengths, int beam, int nbest, int blank, const avctc_ngram_lm* lm,
-                                        double lm_weight, double token_bonus, int32_t* out_tokens, int32_t* out_len,
-                                        double* out_scores, double* out_acoustic, double* out_lm, int32_t* status,
-                                        void* workspace, size_t workspace_bytes, void* stream) {
-    if (N < 0 || T < 0 || V < 1 || beam < 1 || nbest < 1 || nbest > beam || blank < 0 || blank >= V)
-        return AVCTC_ERR_BAD_ARG;
+namespace {
+
+// §4.14's checks of an LM descriptor and its weights.
+bool lm_args_ok(const avctc_ngram_lm* lm, int V, double lm_weight, double token_bonus) {
     if (!lm || lm->order < 1 || lm->order > 5 || lm->map_len != V || !std::isfinite(lm_weight) || lm_weight < 0.0 ||
         !std::isfinite(token_bonus) || lm->num_words < 3 || lm->num_words > 2048 || lm->bos < 0 ||
         lm->bos >= lm->num_words || lm->eos < 0 || lm->eos >= lm->num_words || !lm->token_word || !lm->unigram)
-        return AVCTC_ERR_BAD_ARG;
+        return false;
     for (int o = 2; o <= lm->order; ++o) {
         const uint64_t cap = lm->capacity[o - 2];
-        if (!lm->table[o - 2] || cap < 2 || (cap & (cap - 1))) return AVCTC_ERR_BAD_ARG;
+        if (!lm->table[o - 2] || cap < 2 || (cap & (cap - 1))) return false;
     }
+    return true;
+}
+
+// Both launches of the LM and / or biased search; the arguments are checked by the caller.  lm = NULL gives an
+// unused PbLm of order 1, cx = NULL an unused PbCtx.
+template <bool kLm, bool kBias>
+int launch_lm_search(const float* log_probs, int64_t stride_n, int64_t stride_t, int N, int T, int V,
+                     const int64_t* lengths, int beam, int nbest, int blank, const avctc_ngram_lm* lm,
+                     double lm_weight, double token_bonus, const avctc_context_graph* cx, int32_t* out_tokens,
+                     int32_t* out_len, double* out_scores, double* out_acoustic, double* out_lm, double* out_bias,
+                     int32_t* status, void* workspace, size_t workspace_bytes, void* stream) {
     PbPlan pl;
     if (!pb_plan(N, T, V, beam, &pl)) return AVCTC_ERR_UNSUPPORTED;
     if (N == 0) return AVCTC_OK;
-    if (!out_len || !out_scores || !out_acoustic || !out_lm || !status || !workspace ||
+    if (!out_len || !out_scores || !out_acoustic || !out_lm || (kBias && !out_bias) || !status || !workspace ||
         (T > 0 && (!log_probs || !out_tokens)))
         return AVCTC_ERR_BAD_ARG;
     if (workspace_bytes < pl.total) return AVCTC_ERR_WORKSPACE;
@@ -600,29 +691,78 @@ extern "C" int avctc_ctc_prefix_beam_lm(const float* log_probs, int64_t stride_n
     p.nodes_g = pl.smem_nodes ? nullptr : reinterpret_cast<uint32_t*>(w + pl.off_nodes);
     p.node_cap = pl.node_cap;
     p.out_tokens = out_tokens; p.out_len = out_len; p.out_scores = out_scores; p.status = status;
-    PbLm d;
-    d.token_word = lm->token_word;
-    d.unigram = reinterpret_cast<const float2*>(lm->unigram);
-    for (int o = 0; o < 4; ++o) {
-        const bool used = o + 2 <= lm->order;
-        d.tab[o] = used ? reinterpret_cast<const ulonglong2*>(lm->table[o]) : nullptr;
-        d.mask[o] = used ? lm->capacity[o] - 1 : 0;
+    PbLm d = {};
+    d.order = 1;
+    if (lm) {
+        d.token_word = lm->token_word;
+        d.unigram = reinterpret_cast<const float2*>(lm->unigram);
+        for (int o = 0; o < 4; ++o) {
+            const bool used = o + 2 <= lm->order;
+            d.tab[o] = used ? reinterpret_cast<const ulonglong2*>(lm->table[o]) : nullptr;
+            d.mask[o] = used ? lm->capacity[o] - 1 : 0;
+        }
+        d.order = lm->order; d.bos = lm->bos; d.eos = lm->eos;
+        d.alpha = lm_weight; d.beta = token_bonus;
     }
-    d.order = lm->order; d.bos = lm->bos; d.eos = lm->eos;
-    d.alpha = lm_weight; d.beta = token_bonus;
+    PbCtx c = {};
+    if (cx) {
+        c.token_sym = cx->token_sym;
+        c.delta = cx->delta;
+        c.node = reinterpret_cast<const double2*>(cx->node);
+        c.alphabet = cx->alphabet;
+    }
     const int rc = avctc_beam_topk_lists(log_probs, stride_n, stride_t, N, T, V, lengths, pl.k,
                                          reinterpret_cast<float*>(w + pl.off_tv),
                                          reinterpret_cast<int32_t*>(w + pl.off_ti), stream);
     if (rc) return rc;
-    const size_t per_warp = round_up(kPbLmFixedBytes + (pl.smem_nodes ? (size_t)pl.node_cap * 4 : 0), 16);
+    constexpr size_t fixed = kBias ? kPbBiasFixedBytes : kPbLmFixedBytes;
+    const size_t per_warp = round_up(fixed + (pl.smem_nodes ? (size_t)pl.node_cap * 4 : 0), 16);
     const size_t smem = per_warp * kPbWarps;
     static bool configured = false;
     if (!configured && smem > 48 * 1024) {
-        AVCTC_CUDA_RETURN(cudaFuncSetAttribute(ctc_prefix_beam_lm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                               (int)round_up((size_t)kPbLmFixedBytes + (size_t)kPbSmemNodes * 4, 16) * kPbWarps));
+        AVCTC_CUDA_RETURN(cudaFuncSetAttribute(ctc_prefix_beam_lm_kernel<kLm, kBias>,
+                                               cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               (int)round_up(fixed + (size_t)kPbSmemNodes * 4, 16) * kPbWarps));
         configured = true;
     }
-    ctc_prefix_beam_lm_kernel<<<(N + kPbWarps - 1) / kPbWarps, kPbWarps * 32, smem, reinterpret_cast<cudaStream_t>(stream)>>>(
-        p, d, out_acoustic, out_lm, (int)per_warp);
+    ctc_prefix_beam_lm_kernel<kLm, kBias><<<(N + kPbWarps - 1) / kPbWarps, kPbWarps * 32, smem,
+                                            reinterpret_cast<cudaStream_t>(stream)>>>(
+        p, d, out_acoustic, out_lm, (int)per_warp, c, out_bias);
     return (int)cudaGetLastError();
+}
+
+}  // namespace
+
+extern "C" int avctc_ctc_prefix_beam_lm(const float* log_probs, int64_t stride_n, int64_t stride_t, int N, int T, int V,
+                                        const int64_t* lengths, int beam, int nbest, int blank, const avctc_ngram_lm* lm,
+                                        double lm_weight, double token_bonus, int32_t* out_tokens, int32_t* out_len,
+                                        double* out_scores, double* out_acoustic, double* out_lm, int32_t* status,
+                                        void* workspace, size_t workspace_bytes, void* stream) {
+    if (N < 0 || T < 0 || V < 1 || beam < 1 || nbest < 1 || nbest > beam || blank < 0 || blank >= V)
+        return AVCTC_ERR_BAD_ARG;
+    if (!lm_args_ok(lm, V, lm_weight, token_bonus)) return AVCTC_ERR_BAD_ARG;
+    return launch_lm_search<true, false>(log_probs, stride_n, stride_t, N, T, V, lengths, beam, nbest, blank, lm,
+                                         lm_weight, token_bonus, nullptr, out_tokens, out_len, out_scores,
+                                         out_acoustic, out_lm, nullptr, status, workspace, workspace_bytes, stream);
+}
+
+extern "C" int avctc_ctc_prefix_beam_biased(const float* log_probs, int64_t stride_n, int64_t stride_t, int N, int T,
+                                            int V, const int64_t* lengths, int beam, int nbest, int blank,
+                                            const avctc_ngram_lm* lm, double lm_weight, double token_bonus,
+                                            const avctc_context_graph* ctx, int32_t* out_tokens, int32_t* out_len,
+                                            double* out_scores, double* out_acoustic, double* out_lm, double* out_bias,
+                                            int32_t* status, void* workspace, size_t workspace_bytes, void* stream) {
+    if (N < 0 || T < 0 || V < 1 || beam < 1 || nbest < 1 || nbest > beam || blank < 0 || blank >= V)
+        return AVCTC_ERR_BAD_ARG;
+    if (!ctx || ctx->num_nodes < 1 || ctx->map_len != V || ctx->alphabet < 1 || ctx->alphabet > V ||
+        !ctx->token_sym || !ctx->delta || !ctx->node)
+        return AVCTC_ERR_BAD_ARG;
+    if (lm && !lm_args_ok(lm, V, lm_weight, token_bonus)) return AVCTC_ERR_BAD_ARG;
+    if (lm)
+        return launch_lm_search<true, true>(log_probs, stride_n, stride_t, N, T, V, lengths, beam, nbest, blank, lm,
+                                            lm_weight, token_bonus, ctx, out_tokens, out_len, out_scores,
+                                            out_acoustic, out_lm, out_bias, status, workspace, workspace_bytes, stream);
+    return launch_lm_search<false, true>(log_probs, stride_n, stride_t, N, T, V, lengths, beam, nbest, blank, nullptr,
+                                         0.0, 0.0, ctx, out_tokens, out_len, out_scores, out_acoustic, out_lm,
+                                         out_bias, status, workspace, workspace_bytes, stream);
 }

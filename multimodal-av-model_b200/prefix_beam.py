@@ -1,7 +1,7 @@
 """CTC prefix beam search: ranked transcription hypotheses with their log-probabilities.
 
     ctc_prefix_beam_search(log_probs[N,T,V], lengths=None, beam_width=5, nbest=1, blank=0,
-                           lm=None, lm_weight=0.5, token_bonus=0.0) -> list[list[Hypothesis]]
+                           lm=None, lm_weight=0.5, token_bonus=0.0, context=None) -> list[list[Hypothesis]]
 
 Unlike simple_beam_search, which keeps raw alignment paths and so returns the greedy collapse, the prefix beam search
 scores each prefix by the sum over all of its alignments and merges the alignments that collapse to the same text.
@@ -12,6 +12,10 @@ tensors only.
 With an n-gram LM (ngram_lm.NgramLM), the search fuses it shallowly (DESIGN.md §4.14, oracle/prefix_beam_lm_oracle.py):
 prefixes are ranked by acoustic + lm_weight * ln P_LM + token_bonus * length, </s> included at the end, and each
 hypothesis is an LMHypothesis carrying both parts.
+
+With a phrase list (context_graph.ContextGraph), the search biases towards those phrases (DESIGN.md §4.15,
+oracle/context_graph_oracle.py), with or without an LM: prefixes are ranked by acoustic (+ lm) + bias, a completed
+phrase earns the sum of its per-token weights, and each hypothesis is a BiasedHypothesis.
 """
 from __future__ import annotations
 
@@ -24,6 +28,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from .context_graph import ContextGraph
 from .ngram_lm import NgramLM
 
 MAX_BEAM = 15
@@ -44,12 +49,21 @@ class LMHypothesis(Hypothesis):
     lm_score: float
 
 
+@dataclass
+class BiasedHypothesis(LMHypothesis):
+    """A hypothesis of the biased search: score = (acoustic_score + lm_score) + bias_score, where bias_score is the
+    sum of the per-token weights of every phrase the tokens complete (lm_score is 0.0 without an LM)."""
+    bias_score: float
+
+
 def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: int = 1, blank: int = 0,
-                           lm: NgramLM = None, lm_weight: float = 0.5, token_bonus: float = 0.0) -> List[List[Hypothesis]]:
+                           lm: NgramLM = None, lm_weight: float = 0.5, token_bonus: float = 0.0,
+                           context: ContextGraph = None) -> List[List[Hypothesis]]:
     """log_probs: CUDA [N,T,V] log-probabilities (any float dtype; read as fp32).  lengths: frames to decode per
     utterance (default T).  Returns, per utterance, up to nbest hypotheses, best first.  V <= 1024.  With `lm`, an
     NgramLM built for this model's V pieces, hypotheses are LMHypothesis ranked by the fused score; lm_weight must be
-    finite and >= 0, token_bonus finite."""
+    finite and >= 0, token_bonus finite.  With `context`, a ContextGraph built for V pieces and this blank, hypotheses
+    are BiasedHypothesis ranked by the biased score, with or without `lm`."""
     _lib.require_cuda(log_probs, "log_probs")
     if log_probs.dim() != 3:
         raise RuntimeError("log_probs must be (N, T, V)")
@@ -71,6 +85,13 @@ def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: 
             raise ValueError(f"lm_weight must be finite and >= 0, got {lm_weight}")
         if not math.isfinite(beta):
             raise ValueError(f"token_bonus must be finite, got {token_bonus}")
+    if context is not None:
+        if not isinstance(context, ContextGraph):
+            raise TypeError(f"context must be a ContextGraph, got {type(context).__name__}")
+        if context.vocab_size != V:
+            raise ValueError(f"the context graph was built for {context.vocab_size} pieces, log_probs have V={V} classes")
+        if context.blank != blank:
+            raise ValueError(f"the context graph was built for blank {context.blank}, the search uses blank {blank}")
     lp = log_probs.detach()
     if lp.dtype != torch.float32:
         lp = lp.float()
@@ -87,8 +108,8 @@ def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: 
             raise RuntimeError("lengths must be a 1-D tensor of one entry per utterance")
     Tp = max(T, 1)
     # every output in one device buffer, so that results and statuses come back with one copy; with an LM the scores
-    # are [3][N][nbest]: fused, acoustic, LM
-    nsc = 1 if lm is None else 3
+    # are [3][N][nbest]: fused, acoustic, LM; with a context graph [4][N][nbest]: fused, acoustic, LM, bias
+    nsc = 4 if context is not None else 1 if lm is None else 3
     n_sc, n_len, n_st, n_tok = nsc * N * nbest * 8, N * nbest * 4, N * 4, N * nbest * Tp * 4
     o_len = n_sc
     o_st = o_len + n_len
@@ -100,7 +121,16 @@ def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: 
     tokens = out[o_tok:].view(torch.int32)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
     with _lib.device_guard(dev):
-        if lm is None:
+        if context is not None:
+            sc4 = scores.view(4, N * nbest)
+            _lib.check(L.avctc_ctc_prefix_beam_biased(
+                lp.data_ptr(), lp.stride(0), lp.stride(1), N, T, V, lengths.data_ptr() if lengths is not None else None,
+                B, nbest, blank, ctypes.addressof(lm.descriptor(dev)) if lm is not None else None,
+                alpha if lm is not None else 0.0, beta if lm is not None else 0.0,
+                ctypes.addressof(context.descriptor(dev)), tokens.data_ptr(), lens.data_ptr(), sc4[0].data_ptr(),
+                sc4[1].data_ptr(), sc4[2].data_ptr(), sc4[3].data_ptr(), status.data_ptr(), ws.data_ptr(), ws_bytes,
+                _lib.stream_ptr(dev)), "avctc_ctc_prefix_beam_biased")
+        elif lm is None:
             _lib.check(L.avctc_ctc_prefix_beam(
                 lp.data_ptr(), lp.stride(0), lp.stride(1), N, T, V, lengths.data_ptr() if lengths is not None else None,
                 B, nbest, blank, tokens.data_ptr(), lens.data_ptr(), scores.data_ptr(), status.data_ptr(),
@@ -131,7 +161,10 @@ def ctc_prefix_beam_search(log_probs, lengths=None, beam_width: int = 5, nbest: 
         for i in range(nbest):
             if not sc[n, i] > -np.inf:                    # unused slot
                 break
-            if lm is None:
+            if context is not None:
+                row.append(BiasedHypothesis(tk[n, i, :ln[n, i]].tolist(), float(sc[n, i]), float(sc_all[1, n, i]),
+                                            float(sc_all[2, n, i]), float(sc_all[3, n, i])))
+            elif lm is None:
                 row.append(Hypothesis(tk[n, i, :ln[n, i]].tolist(), float(sc[n, i])))
             else:
                 row.append(LMHypothesis(tk[n, i, :ln[n, i]].tolist(), float(sc[n, i]), float(sc_all[1, n, i]),

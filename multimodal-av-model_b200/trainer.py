@@ -33,6 +33,7 @@ from .beam_search import beam_search_batch, fast_decode
 from .contrastive import contrastive_loss_with_mask
 from .ctc import CTCLoss
 from .ddp import GradBucketReducer, broadcast_buffers, broadcast_module
+from .context_graph import ContextGraph
 from .prefix_beam import ctc_prefix_beam_search
 
 
@@ -491,12 +492,16 @@ class MultimodalTrainer:
         return out
 
     # ------------------------------------------------------------------------------------------ transcription
-    def transcribe(self, batch, beam_width=None, nbest=1, lm=None, lm_weight=0.5, token_bonus=0.0):
+    def transcribe(self, batch, beam_width=None, nbest=1, lm=None, lm_weight=0.5, token_bonus=0.0, context=None):
         """What each speaker said: a CTC prefix beam search over the CTC head's log-probs, computed in eval mode with the
         encoder -> fusion -> decoder1 path that align() uses, decoded on the fusion's input lengths.  The batch needs no
         transcripts.  beam_width defaults to self.beam_width (at most 15).  Returns out[s][b] = [(text, score), ...],
         best first, up to nbest per utterance; score is the hypothesis' natural-log probability, or with `lm` (an
-        NgramLM over this tokenizer's pieces) the fused score acoustic + lm_weight * ln P_LM + token_bonus * length."""
+        NgramLM over this tokenizer's pieces) the fused score acoustic + lm_weight * ln P_LM + token_bonus * length.
+        `context` biases both speakers' searches towards a phrase list: a ContextGraph, or phrase strings encoded with
+        self.tokenizer at the default weight; the score then includes each hypothesis' bias."""
+        if context is not None and not isinstance(context, ContextGraph):
+            context = ContextGraph.from_text(context, self.tokenizer)
         for m in (self.visual_encoder, self.audio_encoder, self.fusion_module, self.decoder1):
             m.eval()
         bw = self.beam_width if beam_width is None else beam_width
@@ -515,7 +520,7 @@ class MultimodalTrainer:
                     fused, il = self.fusion_module(vis, aud, mask_ds)
                     lp = self.decoder1(fused)
                     hyps = ctc_prefix_beam_search(lp, il, beam_width=bw, nbest=nbest, blank=blank, lm=lm,
-                                                  lm_weight=lm_weight, token_bonus=token_bonus)
+                                                  lm_weight=lm_weight, token_bonus=token_bonus, context=context)
                     out.append([[(fast_decode(h.tokens, self.tokenizer), h.score) for h in row] for row in hyps])
         return out
 
