@@ -416,6 +416,12 @@ class AudioEncoder(nn.Module):
 # torch's attention interface between them, called exactly as Wav2Vec2Attention.forward calls it (its dropout stream
 # cannot be reproduced by our own kernel).  The module path stays the reference and the path for everything else.
 
+def _w2v_native_shape_ok(m, e, f):
+    """The shapes csrc/wav2vec2_layer.cu takes: rows m > 0, hidden e a multiple of 256 up to 1024, intermediate f a
+    positive multiple of 8."""
+    return m > 0 and 0 < e <= 1024 and e % 256 == 0 and f > 0 and f % 8 == 0
+
+
 def _w2v_native_applies(layer, hidden):
     """bf16-autocast CUDA forward of a Wav2Vec2EncoderLayerStableLayerNorm with sdpa attention, exact GELU, no adapter,
     fp32 parameters and dropout probabilities below 1, outside stream capture."""
@@ -430,7 +436,7 @@ def _w2v_native_applies(layer, hidden):
     if getattr(cfg, "_attn_implementation", None) != "sdpa" or cfg.hidden_act != "gelu":
         return False
     e, f = hidden.shape[-1], layer.feed_forward.intermediate_dense.out_features
-    if e % 256 or e > 1024 or f % 8 or hidden.shape[0] * hidden.shape[1] == 0:
+    if not _w2v_native_shape_ok(hidden.shape[0] * hidden.shape[1], e, f):
         return False
     ff = layer.feed_forward
     if any(not 0.0 <= d.p < 1.0 for d in (layer.dropout, ff.intermediate_dropout, ff.output_dropout)):

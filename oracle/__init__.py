@@ -16,6 +16,8 @@ Layers:
   * ``np_oracle.py``   numpy float64 restatement of fusion_module / decoder / contrastive arithmetic.
   * ``torch_port.py``  restatement of the same modules on torch CPU ops (what the reference really
     executes); used for gradients at larger sizes and as the timed CPU baseline.
+  * ``w2v_oracle.py``  float64 forward and backward of the two wav2vec2 layer halves csrc/wav2vec2_layer.cu runs,
+    written out without autograd, with optional bf16 rounding at the module path's points.
 """
 from __future__ import annotations
 

@@ -22,10 +22,10 @@ def _gen():
     return torch.cuda.default_generators[torch.cuda.current_device()]
 
 
-def _layer(seed=0, trainable=True, train=True):
+def _layer(seed=0, trainable=True, train=True, **cfg_overrides):
     from transformers.models.wav2vec2.modeling_wav2vec2 import Wav2Vec2EncoderLayerStableLayerNorm
     from multimodal_av_model_b200.encoders import xlsr_large_config
-    cfg = xlsr_large_config()
+    cfg = xlsr_large_config(**cfg_overrides)
     cfg._attn_implementation = "sdpa"
     torch.manual_seed(seed)
     layer = Wav2Vec2EncoderLayerStableLayerNorm(cfg).cuda()
@@ -37,9 +37,9 @@ def _layer(seed=0, trainable=True, train=True):
     return layer.train(train)
 
 
-def _inputs(seed=1):
+def _inputs(seed=1, e=1024):
     g = torch.Generator(device="cuda").manual_seed(seed)
-    x = torch.randn(B, T, 1024, device="cuda", generator=g).to(torch.bfloat16)
+    x = torch.randn(B, T, e, device="cuda", generator=g).to(torch.bfloat16)
     lens = torch.tensor([249, 200, 131, 249, 17, 90, 248, 160])
     m = torch.arange(T)[None, :] < lens[:, None]
     x = x.masked_fill(~m.cuda()[..., None], 0)                                   # padded frames are 0, as upstream
@@ -115,6 +115,19 @@ def test_native_layer_matches_module_path_train(trainable):
     _close(y, z, "y", rel=1e-2)
     _close(dx, dx_ref, "dx")
     assert (len(g) == 16) == trainable
+    _grads_close(g, g_ref, 3e-2)
+
+
+def test_native_layer_matches_module_path_train_768():
+    """A 768-wide layer (a base model's width) takes the native path too: three 256-column chunks per LayerNorm row."""
+    layer = _layer(7, hidden_size=768, intermediate_size=3072, num_attention_heads=12)
+    x, mask4d = _inputs(7, e=768)
+    y, off, dx, g = _run(layer, x, mask4d, native=True)
+    z, off_ref, dx_ref, g_ref = _run(layer, x, mask4d, native=False)
+    assert off == off_ref
+    _close(y, z, "y", rel=1e-2)
+    _close(dx, dx_ref, "dx")
+    assert len(g) == 16
     _grads_close(g, g_ref, 3e-2)
 
 
