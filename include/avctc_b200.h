@@ -297,7 +297,8 @@ AVCTC_API int avctc_resample_backward(const void* dout_bf16, int B, int Ta, int 
 AVCTC_API int avctc_softmax_forward(const float* S, void* P_bf16, long long rows, int T, int Tp, void* stream);
 AVCTC_API int avctc_softmax_backward(const void* P_bf16, const float* dP, void* dS_bf16, long long rows, int T, int Tp,
                            void* stream);
-/* out[n] (+)= sum_m X[m*ld + n]  (bias gradients). */
+/* out[n] (+)= sum_m X[m*ld + n]  (bias gradients).  ld >= N; AVCTC_ERR_BAD_ARG otherwise, and for a bad dtype, with
+ * out left untouched. */
 AVCTC_API int avctc_colsum(const void* X, int dtype, long long M, int N, long long ld, float* out, int accumulate,
                  void* stream);
 /* CTC head: F.log_softmax over V classes (/root/reference/model/decoder.py:25) and its backward

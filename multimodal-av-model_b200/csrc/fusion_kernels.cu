@@ -340,6 +340,7 @@ extern "C" int avctc_resample_forward(const void* audio, int dtype, const int64_
     if (B <= 0 || Ta <= 0 || D <= 0 || Tv <= 0) return AVCTC_ERR_BAD_ARG;
     if (!audio || !mask || !out_bf16 || !mask_out || !input_lengths || !workspace) return AVCTC_ERR_BAD_ARG;
     if (workspace_bytes < avctc_resample_workspace_bytes(B, Ta)) return AVCTC_ERR_WORKSPACE;
+    if (dtype != AVCTC_F32 && dtype != AVCTC_BF16) return AVCTC_ERR_BAD_ARG;
     if ((D & 7) == 0 && ((reinterpret_cast<uintptr_t>(audio) | reinterpret_cast<uintptr_t>(out_bf16)) & 15))
         return AVCTC_ERR_ALIGNMENT;      // the 8-wide path uses 16-byte accesses
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
@@ -358,7 +359,6 @@ extern "C" int avctc_resample_forward(const void* audio, int dtype, const int64_
                                                                   Ta, D, Tv, src, cnt,
                                                                   reinterpret_cast<__nv_bfloat16*>(out_bf16), mask_out,
                                                                   input_lengths);
-    else return AVCTC_ERR_BAD_ARG;
     return (int)cudaGetLastError();
 }
 
@@ -398,7 +398,8 @@ extern "C" int avctc_softmax_backward(const void* P_bf16, const float* dP, void*
 
 extern "C" int avctc_colsum(const void* X, int dtype, long long M, int N, long long ld, float* out, int accumulate,
                             void* stream) {
-    if (!X || !out || M <= 0 || N <= 0) return AVCTC_ERR_BAD_ARG;
+    if (!X || !out || M <= 0 || N <= 0 || ld < N) return AVCTC_ERR_BAD_ARG;
+    if (dtype != AVCTC_F32 && dtype != AVCTC_BF16) return AVCTC_ERR_BAD_ARG;   // before the memset: out stays intact
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     int chunks = (int)((M + 127) / 128);
     if (chunks > 64) chunks = 64;
@@ -407,7 +408,6 @@ extern "C" int avctc_colsum(const void* X, int dtype, long long M, int N, long l
     if (dtype == AVCTC_F32) colsum_kernel<float><<<grid, 256, 0, st>>>(reinterpret_cast<const float*>(X), M, N, ld, out);
     else if (dtype == AVCTC_BF16)
         colsum_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat16*>(X), M, N, ld, out);
-    else return AVCTC_ERR_BAD_ARG;
     return (int)cudaGetLastError();
 }
 

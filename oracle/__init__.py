@@ -18,6 +18,8 @@ Layers:
     executes); used for gradients at larger sizes and as the timed CPU baseline.
   * ``w2v_oracle.py``  float64 forward and backward of the two wav2vec2 layer halves csrc/wav2vec2_layer.cu runs,
     written out without autograd, with optional bf16 rounding at the module path's points.
+  * ``fusion_oracle.py``  float64 forward and backward of the fusion-path kernels (resample, softmax, column sums,
+    log-softmax, attention, GEMM), with optional bf16 rounding where the attention kernel materialises bf16.
 """
 from __future__ import annotations
 
